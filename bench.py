@@ -8,11 +8,15 @@ decode -> channelise -> detect -> integrate -> rescale -> requantise -> splice) 
 60 s scan.  `value` is measured with the VDIF already in HBM; `e2e` pushes the same scan from
 pinned host memory through the C ABI and reads the finished rows back to the host.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--seconds S] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--seconds S] [--impl reference] [--dump-outputs DIR]
 
 N > 1: launched under torch.distributed.run, one rank per GPU; every rank processes its own
 8-IF band (weak scaling: N x 8 subbands) and the finished 8-bit tiles are gathered over NCCL
 into rank 0's band-ordered rows -- the one exchange the path has (base2fil.sh:422).
+
+--dump-outputs DIR (one GPU): after the timed steps, write what the last of them delivered as float32
+.npy files (see dump_outputs).  The input is generated from fixed seeds, so two builds run with the
+same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -106,6 +110,27 @@ def make_device_vdif(torch, dev, nframes: int, seed: int):
     return out
 
 
+#: size limit of the rows --dump-outputs writes as float32; longer outputs are dumped as a seeded sample of whole rows
+DUMP_ROW_BYTES = 48 << 20
+
+
+def dump_outputs(path: str, torch, plan, out_dev, rows: int):
+    """The outputs of the last timed step as float32 .npy files in `path`:
+    rows.npy         the spliced output rows in their sample values ([n, channels x products]); all `rows` of them, or n of
+                     them chosen with a fixed seed when all would exceed DUMP_ROW_BYTES
+    row_index.npy    which rows those are (float64), so that a build producing a different row count shows up
+    rescale_mean.npy, rescale_scale.npy   the requantiser's statistics the step measured ([nif, products, nchan])"""
+    os.makedirs(path, exist_ok=True)
+    elems = plan.view_rows(np.empty((0, int(plan.row_bytes)), np.uint8)).shape[1]
+    n = min(rows, max(1, DUMP_ROW_BYTES // (4 * elems)))
+    idx = np.arange(rows) if n == rows else np.sort(np.random.default_rng(20121102).choice(rows, n, replace=False))
+    sample = out_dev[torch.from_numpy(idx).to(out_dev.device)].cpu().numpy()
+    mean, scale = plan.rescale()
+    for name, a in (("rows", plan.view_rows(sample)), ("row_index", idx.astype(np.float64)),
+                    ("rescale_mean", mean), ("rescale_scale", scale)):
+        np.save(os.path.join(path, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons during the timed region (B200_PROFILING.md)."""
     Q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
@@ -179,8 +204,9 @@ def _cpu_worker(args):
     return time.perf_counter() - t0, r["data"].shape[0]
 
 
-def cpu_arm(cfg: dict, sample_seconds: float, steps: int = 1):
-    """Time the oracle (CPU restatement of digifil+splice) on this box's host cores."""
+def cpu_arm(cfg: dict, sample_seconds: float, steps: int = 1, warmup: int = 0):
+    """Time the oracle (CPU restatement of digifil+splice) on the host's cores: `warmup` untimed passes, then the median
+    of `steps` timed ones."""
     import multiprocessing as mp
     from frb_baseband_b200 import synth
     cores = len(os.sched_getaffinity(0))
@@ -193,11 +219,12 @@ def cpu_arm(cfg: dict, sample_seconds: float, steps: int = 1):
     ctx = mp.get_context("spawn")      # the parent may hold a CUDA context: never fork it
     times = []
     with ctx.Pool(workers) as pool:
-        for _ in range(steps):
+        for k in range(warmup + steps):
             res = pool.map(_cpu_worker, jobs)
             # splice: concatenate per-IF rows, highest frequency first (trivial next to digifil)
             wall = max(r[0] for r in res) if workers >= NIF else sum(r[0] for r in res) / workers
-            times.append(max(wall, 1e-9))
+            if k >= warmup:
+                times.append(max(wall, 1e-9))
     t = float(np.median(times))
     data_sec = nframes / FPS
     return {"value": NIF * nframes * FRAME_BYTES / t / 1e9, "unit": "GB/s", "cores": workers * nthr, "kind": "port",
@@ -249,7 +276,11 @@ def main():
     ap.add_argument("--chunk-units", type=int, default=4, help="frames per push in units of whole-block frame groups (0 = library default)")
     ap.add_argument("--nccl-gather", action="store_true", help="splice with an NCCL gather instead of peer stores")
     ap.add_argument("--cpu-sample", type=float, default=1.024, help="seconds of data for the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR as float32 .npy files (one GPU only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = select_config(args.config)
     seconds = args.seconds if args.seconds else cfg.get("sample_seconds", cfg["seconds"])
     workload = cfg["what"].format(sec=seconds)
@@ -257,12 +288,14 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (world > 1 or args.impl != "b2f"):
+        ap.error("--dump-outputs dumps the b2f path of a one-GPU run")
 
     if args.impl == "reference":
         if rank != 0:
             return 0
         W = max(args.warmup, 0)
-        r = cpu_arm(cfg, args.cpu_sample, steps=max(1, args.steps + min(W, 1)))
+        r = cpu_arm(cfg, args.cpu_sample, steps=args.steps, warmup=min(W, 1))
         line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "GB/s", "n_gpus": args.gpus,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["seconds_per_step"] * 1e3,
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -380,6 +413,8 @@ def main():
     ms_step, rows, launches, (t0, t1) = timed(pl, step_device, args.steps, max(args.warmup, 3))
     clocks = sampler.stop(t0, t1)
     ktimes = pl.kernel_times()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, torch, pl, out_dev, int(rows))
     data_sec = nframes / FPS
     in_bytes = NIF * nframes * FRAME_BYTES
     value = world * in_bytes / (ms_step * 1e-3) / 1e9
@@ -400,7 +435,7 @@ def main():
             except Exception:
                 peers = None
         step_s, _ = make_step(pls, vd[:per], outs, peers)
-        ms_s, rows_s, _, _ = timed(pls, step_s, max(1, min(args.steps, 3)), 2)
+        ms_s, rows_s, _, _ = timed(pls, step_s, args.steps, 2)
         strong = {"ifs_per_gpu": per, "ms_per_step": ms_s, "value": in_bytes / (ms_s * 1e-3) / 1e9, "unit": "GB/s",
                   "rt_factor": data_sec / (ms_s * 1e-3), "efficiency_vs_this_runs_weak_per_gpu_rate": ms_step / (world * ms_s),
                   "chunk_frames": int(pls.chunk_frames), "rows_per_step": int(rows_s),
@@ -437,7 +472,7 @@ def main():
             pl.sync()
             return got
 
-        ms_e2e, rows_e, _, _ = timed(pl, step_host, max(1, min(args.steps, 3)), 1)
+        ms_e2e, rows_e, _, _ = timed(pl, step_host, args.steps, 1)
         h2d = sum(n for _, n in chunks) * NIF * FRAME_BYTES
         # the ceiling of that number: a bare pinned-host -> device copy of the same buffers (PCIe), nothing else
         scratch = torch.empty_like(vd[0][:hold_frames])
