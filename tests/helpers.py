@@ -29,12 +29,22 @@ def assert_rel(gpu, ref, tol=REL_TOL, what="", power=None):
 
 
 def run_plan(vdifs, *, nchan, bw, tscrunch=1, pol_mode=_lib.POL_I, out_nbit=8, in_nbit=2, keep_bandpass=False,
-             freq=None, interval=10.0, chunk_frames=None, splice_pol_major=False, profile=False):
-    """Push a list of per-IF VDIF arrays through a Plan chunk by chunk; return (rows, plan info)."""
+             freq=None, interval=10.0, chunk_units=0, splice_pol_major=False, profile=False, **cfg_kw):
+    """Push a list of per-IF VDIF arrays through a Plan chunk by chunk; return (rows, plan info).  `chunk_units`
+    sets the push size (PlanConfig.chunk_units, 0 = the library default); other PlanConfig fields go in `cfg_kw`.
+    Every pull is repeated until it returns nothing: the running rescale mode hands out one interval per pull."""
     cfg = PlanConfig(nchan=nchan, bw_mhz=list(bw), freq_mhz=freq, tscrunch=tscrunch, pol_mode=pol_mode,
-                     out_nbit=out_nbit, in_nbit=in_nbit, keep_bandpass=keep_bandpass,
-                     rescale_interval_s=interval, splice_pol_major=splice_pol_major, profile=profile)
+                     out_nbit=out_nbit, in_nbit=in_nbit, keep_bandpass=keep_bandpass, chunk_units=chunk_units,
+                     rescale_interval_s=interval, splice_pol_major=splice_pol_major, profile=profile, **cfg_kw)
     out = []
+
+    def drain(pl):
+        while True:
+            r = pl.pull()
+            if not len(r):
+                return
+            out.append(r.copy())
+
     with Plan(cfg) as pl:
         fb = cfg.frame_bytes
         nfr = min(v.size // fb for v in vdifs)
@@ -42,14 +52,11 @@ def run_plan(vdifs, *, nchan, bw, tscrunch=1, pol_mode=_lib.POL_I, out_nbit=8, i
         for f0 in range(0, nfr, cf):
             n = min(cf, nfr - f0)
             pl.push([v[f0 * fb:(f0 + n) * fb] for v in vdifs])
-            r = pl.pull()
-            if len(r):
-                out.append(r.copy())
+            drain(pl)
         pl.flush()
-        r = pl.pull()
-        if len(r):
-            out.append(r.copy())
-        info = {"counters": pl.counters(), "rescale": pl.rescale(), "geometry": pl.geometry,
-                "nprod": pl.nprod, "if_order": pl.if_order, "times": pl.kernel_times() if profile else None}
+        drain(pl)
+        info = {"counters": pl.counters(), "rescale": pl.rescale(), "geometry": pl.geometry, "path": pl.path,
+                "chunk_frames": int(cf), "nprod": pl.nprod, "if_order": pl.if_order,
+                "times": pl.kernel_times() if profile else None}
         rows = pl.view_rows(np.concatenate(out)) if out else np.empty((0, pl.row_bytes), np.uint8)
     return rows, info

@@ -65,7 +65,7 @@ def test_fused_many_rounds_multi_if_8bit(gpu, monkeypatch):
     nchan, bw, D, nif = 128, 32.0, 16, 8
     vs = [synth.make_vdif(3 * 1024, seed=500 + i, bw_mhz=bw, tone_frac=0.1 * (i + 1)) for i in range(nif)]
     bws = [bw if i % 2 else -bw for i in range(nif)]
-    kw = dict(nchan=nchan, bw=bws, tscrunch=D, interval=0.4, chunk_frames=None)
+    kw = dict(nchan=nchan, bw=bws, tscrunch=D, interval=0.4)
     leg, _ = _rows(monkeypatch, "legacy", vs, **kw)
     f1, _ = _rows(monkeypatch, "fused", vs, **kw)
     f2, _ = _rows(monkeypatch, "fused", vs, **kw)
