@@ -81,8 +81,6 @@ struct b2f_plan {
     double2* d_partial = nullptr;
     float2 *d_tab_g = nullptr, *d_tab_h = nullptr, *d_tab_w = nullptr, *d_tab_r = nullptr, *d_tab_beta = nullptr;
     unsigned long long* d_counters = nullptr;
-    int* d_sm_slots = nullptr;
-    int stagger_cycles = 0;
     int64_t batch_blocks = 0;      // FFT blocks per column/row launch pair (0 = whole chunk)
     // coherent dedispersion (digifil -D dm -F nchan:D): overlap-save geometry and halo carry
     bool dedisp = false;
@@ -120,7 +118,7 @@ struct b2f_plan {
     float* d_part = nullptr;       int64_t part_if_stride = 0;  // partial rows when tscrunch > 1024 / R
     int Dp = 0;                    // rows a warp integrates itself
     unsigned* d_fsync = nullptr;   // per-lane arrival counters + abort flag (last word)
-    int f_grid = 0, f_lanes = 0, f_nslot = 3, f_lag = 2;
+    int f_grid = 0, f_lanes = 0, f_nslot = 3, f_lag = 2;        // fused ring: rows run 2 blocks behind the columns, 3 slots per lane
     bool f_aborted = false;
     float4* d_levels = nullptr;                                 // JA98 decode: output magnitudes per window of 512 samples
     unsigned long long* d_fprof = nullptr;                      // B2F_FUSED_PROF=1: per-warp cycle breakdown of the fused kernel
@@ -209,9 +207,9 @@ int launch_kb(b2f_plan* pl, const KBParams& kp, int grid) {
     return 0;
 }
 
-int launch_ka(b2f_plan* pl, const KAParams& ka, unsigned grid) {
+int launch_ka(b2f_plan* pl, bool fwd_only, const KAParams& ka, unsigned grid) {
     cudaError_t e = cudaSuccess;
-    int rc = timed(pl, B2F_K_COLUMN, [&] { e = b2f_launch_ka(pl->d_levels_stream ? 22 : pl->prm.in_nbit, pl->R, ka, grid, pl->stream); });
+    int rc = timed(pl, B2F_K_COLUMN, [&] { e = b2f_launch_ka(pl->d_levels_stream ? 22 : pl->prm.in_nbit, pl->R, fwd_only, ka, grid, pl->stream); });
     if (rc) return rc;
     if (e != cudaSuccess) return fail(B2F_ECUDA, std::string("column pass launch: ") + cudaGetErrorString(e));
     return 0;
@@ -282,8 +280,7 @@ int launch_k0(b2f_plan* pl, const K0Params& kp, cudaStream_t st, bool profile_ok
     for (int i = 0; i < nif; ++i) aligned = aligned && ((reinterpret_cast<uintptr_t>(kp.frames[i]) & 15) == 0);
     const int stage_bytes = (kp.frame_bytes + 127) & ~127;
     int sms = pl ? pl->num_sms : 148;
-    static const int per_sm = [] { const char* e = getenv("B2F_K0_CTAS_PER_SM"); return e ? std::max(1, atoi(e)) : 4; }();
-    int gx = (int)std::max<int64_t>(1, std::min<int64_t>(kp.nframes, (per_sm * sms + nif - 1) / nif));
+    int gx = (int)std::max<int64_t>(1, std::min<int64_t>(kp.nframes, (kK0CtasPerSM * sms + nif - 1) / nif));
     dim3 grid(gx, nif);
     auto body = [&] {
         if (vec && aligned) {
@@ -319,7 +316,7 @@ void free_plan(b2f_plan* pl) {
             if (pl->ev_mark[i][k]) cudaEventDestroy(pl->ev_mark[i][k]);
     void* bufs[] = {pl->d_compact, pl->d_wmask, pl->d_fstat, pl->d_blkdirty, pl->d_inter, pl->d_colsum,
                     pl->d_eps, pl->d_F, pl->d_mean, pl->d_scale, pl->d_partial, pl->d_tab_g, pl->d_tab_h,
-                    pl->d_tab_w, pl->d_tab_r, pl->d_tab_beta, pl->d_counters, pl->d_sm_slots, pl->d_carry, pl->d_spec, pl->d_chirp, pl->d_tw_col, pl->d_tw_row,
+                    pl->d_tab_w, pl->d_tab_r, pl->d_tab_beta, pl->d_counters, pl->d_carry, pl->d_spec, pl->d_chirp, pl->d_tw_col, pl->d_tw_row,
                     pl->d_tstream, pl->d_fillflag, pl->d_part, pl->d_fsync, pl->d_fprof, pl->d_levels, pl->d_carry_mask, pl->d_levels_stream};
     for (void* b : bufs)
         if (b) cudaFree(b);
@@ -501,7 +498,6 @@ int push_dedisp(b2f_plan* pl, int64_t nblk, int64_t T) {
         ka.in8_offset = pl->prm.in8_offset_mode ? 128.0f : 127.5f;
         ka.levels = pl->d_levels_stream; ka.levels_stride = pl->levels_stride;
         if (int rcl = stream_levels(pl, T)) return rcl;
-        ka.sm_slots = pl->d_sm_slots; ka.stagger_cycles = 0; ka.variant = 32;      // forward only
         KBParams kb{};
         kb.inter = pl->d_inter; kb.eps = nullptr; kb.tab_r = pl->d_tab_r; kb.spec = pl->d_spec;
         kb.F = nullptr; kb.nblk = (int)nblk; kb.nif = nif; kb.D = 1;
@@ -518,7 +514,7 @@ int push_dedisp(b2f_plan* pl, int64_t nblk, int64_t T) {
             ka.gb_begin = b0; ka.gb_end = b0 + nb;
             int64_t grid = std::max<int64_t>(1, (kKACtasPerSM * pl->num_sms) / pl->nstrips) * pl->nstrips;
             grid = std::min<int64_t>(grid, nb * pl->nstrips);
-            rc = launch_ka(pl, ka, (unsigned)grid);
+            rc = launch_ka(pl, true, ka, (unsigned)grid);         // forward only: the chirp goes between row FFT and backward FFT
             if (rc) return rc;
             kb.gb_begin = b0; kb.gb_end = b0 + nb;
             const int64_t ngroups = nb * (kL / RW);
@@ -549,13 +545,12 @@ int push_dedisp(b2f_plan* pl, int64_t nblk, int64_t T) {
     return 0;
 }
 
-cudaError_t b2f_launch_ka(int in_nbit, int R, const KAParams& p, unsigned grid, cudaStream_t st) {
-    if (in_nbit == 22) return b2f_launch_ka_22(R, p, grid, st);                               // 2-bit input, JA98 levels
-    return in_nbit == 8 ? b2f_launch_ka_8(R, p, grid, st) : b2f_launch_ka_2(R, p, grid, st);   // 1- and 2-bit: index-byte stream
+cudaError_t b2f_launch_ka(int in_nbit, int R, bool fwd_only, const KAParams& p, unsigned grid, cudaStream_t st) {
+    if (in_nbit == 22) return b2f_launch_ka_22(R, fwd_only, p, grid, st);                                         // 2-bit input, JA98 levels
+    return in_nbit == 8 ? b2f_launch_ka_8(R, fwd_only, p, grid, st) : b2f_launch_ka_2(R, fwd_only, p, grid, st);   // 1- and 2-bit: index-byte stream
 }
-cudaError_t b2f_launch_kr(int R, int mode, const KBParams& p, int grid, cudaStream_t st) {
+cudaError_t b2f_launch_kr(int R, int mode, const KBParams& p, int grid, cudaStream_t st) {     // R != 256: that row length uses the tile row pass
     if (R <= 64) return b2f_launch_kr_part0(R, mode, p, grid, st);
-    if (R == 256) return b2f_launch_kr_part2(R, mode, p, grid, st);
     return b2f_launch_kr_part1(R, mode, p, grid, st);
 }
 cudaError_t b2f_launch_kb(int R, int mode, const KBParams& p, int grid, cudaStream_t st) {
@@ -699,7 +694,7 @@ int push_fused(b2f_plan* pl, const K0Params& k0, int64_t nframes, int64_t nblk) 
             ke_eps<<<(unsigned)nbt, std::min(pl->R / 2, 512), pl->R * sizeof(float2), pl->stream>>>(pl->d_colsum, pl->d_eps, pl->R);
         });
         if (rc) return rc;
-        if (pl->R == 256 && !getenv("B2F_NO_TILE_ROWS")) {
+        if (pl->R == 256) {
             // 16-row tiles are 32 KiB contiguous in the block layout: one bulk copy per tile, block-wide second FFT stage
             KTParams kt{};
             kt.inter = pl->d_inter; kt.eps = pl->d_eps; kt.tab_r = pl->d_tab_r;
@@ -920,11 +915,9 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     if (dedisp && prm->chunk_units <= 0) {
         // the three-kernel dedispersion path holds two [blocks][512][R] buffers: pushes of about 4096 frames per IF (C4, 20 s:
         // 139.8 ms at 1024 frames, 134.9 at 2048, 134.0 at 4096; profiles/r02_c4_push_size_sweep.jsonl) as long as each buffer
-        // stays under 8 GiB.  B2F_DEDISP_CHUNK_FRAMES overrides.
-        const char* e = getenv("B2F_DEDISP_CHUNK_FRAMES");
-        const int64_t want = e ? std::max<int64_t>(256, atoll(e)) : 4096;
+        // stays under 8 GiB.
         const int64_t unit_bytes = (int64_t)prm->nif * (pl->unit_blocks + 1) * L * R * (int64_t)sizeof(float2);
-        cu = (int)std::max<int64_t>(1, std::min<int64_t>(want / pl->unit_frames, (8ll << 30) / std::max<int64_t>(unit_bytes, 1)));
+        cu = (int)std::max<int64_t>(1, std::min<int64_t>(4096 / pl->unit_frames, (8ll << 30) / std::max<int64_t>(unit_bytes, 1)));
     }
     if (generic) {                 // blocks span seconds: pushes are plain 1024-frame pieces, the carry does the rest
         pl->unit_frames = 1;
@@ -992,9 +985,6 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
                 pl->f_grid = pl->num_sms;                                  // one 16-warp CTA per SM
                 pl->f_lanes = pl->f_grid * kFWarps / npair;
                 if (pl->f_lanes < 1) pl->path = 0;
-                const char* lg = getenv("B2F_ROW_LAG");
-                pl->f_lag = lg ? std::max(2, std::min(3, atoi(lg))) : 2;
-                { const char* e2 = getenv("B2F_RING_SLOTS"); pl->f_nslot = e2 ? std::max(pl->f_lag + 1, std::min(6, atoi(e2))) : pl->f_lag + 1; }
                 pl->Dp = std::min(D, 1024 / R);
             }
         }
@@ -1067,7 +1057,6 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     CUB(cudaMalloc(&pl->d_scale, (size_t)nif * nprod * pl->N * sizeof(float)));
     CUB(cudaMalloc(&pl->d_partial, (size_t)nif * kStatSplit * nprod * pl->N * sizeof(double2)));
     CUB(cudaMalloc(&pl->d_counters, C_COUNT * sizeof(unsigned long long)));
-    CUB(cudaMalloc(&pl->d_sm_slots, 1024 * sizeof(int)));
     if (pl->carry_mode) CUB(cudaMalloc(&pl->d_carry, (size_t)pl->M * pl->bps * nif));
     if (pl->smask) CUB(cudaMalloc(&pl->d_carry_mask, (size_t)pl->M * pl->bps / 32 * nif));
     if (prm->decode_mode == B2F_DECODE_JA98 && (generic || pl->path == 0)) {
@@ -1129,11 +1118,6 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
         }
         CUB(cudaMalloc(&pl->d_chirp, h.size() * sizeof(float2)));
         CUB(cudaMemcpy(pl->d_chirp, h.data(), h.size() * sizeof(float2), cudaMemcpyHostToDevice));
-    }
-    CUB(cudaMemset(pl->d_sm_slots, 0, 1024 * sizeof(int)));
-    {
-        const char* e = getenv("B2F_STAGGER");
-        pl->stagger_cycles = e ? atoi(e) : 0;
     }
 #undef CUB
     int rc = upload_tables(pl);
@@ -1357,14 +1341,9 @@ int b2f_push(b2f_plan* pl, const void* const* frames, int64_t nframes, int on_de
         ka.R = pl->R; ka.nstrips = pl->nstrips; ka.nblk = (int)nblk; ka.nif = nif;
         ka.payload_bytes = (int)pl->payload; ka.groups_per_slot = (int)pl->groups_per_slot;
         ka.blk_step_bytes = pl->M * pl->bps;
-        ka.sm_slots = pl->d_sm_slots; ka.stagger_cycles = pl->stagger_cycles;
         ka.in8_offset = pl->prm.in8_offset_mode ? 128.0f : 127.5f;
         ka.levels = pl->d_levels_stream; ka.levels_stride = pl->levels_stride;
         if (int rcl = stream_levels(pl, T)) return rcl;
-        {
-            const char* e = getenv("B2F_KA_VARIANT");      // timing ablations only (tools/ablate.py)
-            ka.variant = e ? atoi(e) : 0;
-        }
         KBParams kb{};
         kb.inter = pl->d_inter; kb.eps = pl->d_eps; kb.tab_r = pl->d_tab_r;
         kb.F = row_dst(pl); kb.F_if_stride = row_dst_stride(pl);
@@ -1376,7 +1355,7 @@ int b2f_push(b2f_plan* pl, const void* const* frames, int64_t nframes, int on_de
             const int64_t work = nb * pl->nstrips;
             int64_t grid = std::max<int64_t>(1, (kKACtasPerSM * pl->num_sms) / pl->nstrips) * pl->nstrips;
             grid = std::min<int64_t>(grid, work);
-            rc = launch_ka(pl, ka, (unsigned)grid);
+            rc = launch_ka(pl, false, ka, (unsigned)grid);
             if (rc) return rc;
             rc = timed(pl, B2F_K_EPS, [&] {
                 ke_eps<<<(unsigned)nb, std::min(pl->R / 2, 512), pl->R * sizeof(float2), pl->stream>>>(pl->d_colsum + b0 * pl->R,

@@ -6,49 +6,34 @@ using namespace b2f;
 #define B2F_CAT2(a, b) a##b
 #define B2F_CAT(a, b) B2F_CAT2(a, b)
 
-template <int R, int VAR = 0>
+template <int R, bool FWD_ONLY>
 static cudaError_t go(const KAParams& p, unsigned grid, cudaStream_t st) {
-    auto kern = ka_column_pass<B2F_NBIT, R, VAR>;
+    auto kern = ka_column_pass<B2F_NBIT, R, FWD_ONLY>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)KASmem<B2F_NBIT>::kBytes);
     if (e != cudaSuccess) return e;
     kern<<<grid, kKAThreads, KASmem<B2F_NBIT>::kBytes, st>>>(p);
     return cudaGetLastError();
 }
 
-cudaError_t B2F_CAT(b2f_launch_ka_, B2F_NBIT)(int R, const KAParams& p, unsigned grid, cudaStream_t st) {
-#if B2F_NBIT == 2
-    if (R == 256 && p.variant) {               // timing ablations, tools/ablate.py
-        switch (p.variant) {
-            case 1: return go<256, 1>(p, grid, st);
-            case 2: return go<256, 2>(p, grid, st);
-            case 3: return go<256, 3>(p, grid, st);
-            case 4: return go<256, 4>(p, grid, st);
-            case 7: return go<256, 7>(p, grid, st);
-            case 8: return go<256, 8>(p, grid, st);
-            case 15: return go<256, 15>(p, grid, st);
-            case 16: return go<256, 16>(p, grid, st);
-            case 23: return go<256, 23>(p, grid, st);
-        }
-    }
-#endif
-    if (p.variant == 32) {                     // forward-only product mode of the dedispersion path
+cudaError_t B2F_CAT(b2f_launch_ka_, B2F_NBIT)(int R, bool fwd_only, const KAParams& p, unsigned grid, cudaStream_t st) {
+    if (fwd_only) {                            // forward-only product mode of the dedispersion path
         switch (R) {
-            case 16: return go<16, 32>(p, grid, st);
-            case 32: return go<32, 32>(p, grid, st);
-            case 64: return go<64, 32>(p, grid, st);
-            case 128: return go<128, 32>(p, grid, st);
-            case 256: return go<256, 32>(p, grid, st);
-            case 512: return go<512, 32>(p, grid, st);
+            case 16: return go<16, true>(p, grid, st);
+            case 32: return go<32, true>(p, grid, st);
+            case 64: return go<64, true>(p, grid, st);
+            case 128: return go<128, true>(p, grid, st);
+            case 256: return go<256, true>(p, grid, st);
+            case 512: return go<512, true>(p, grid, st);
         }
         return cudaErrorInvalidValue;
     }
     switch (R) {
-        case 16: return go<16>(p, grid, st);
-        case 32: return go<32>(p, grid, st);
-        case 64: return go<64>(p, grid, st);
-        case 128: return go<128>(p, grid, st);
-        case 256: return go<256>(p, grid, st);
-        case 512: return go<512>(p, grid, st);
+        case 16: return go<16, false>(p, grid, st);
+        case 32: return go<32, false>(p, grid, st);
+        case 64: return go<64, false>(p, grid, st);
+        case 128: return go<128, false>(p, grid, st);
+        case 256: return go<256, false>(p, grid, st);
+        case 512: return go<512, false>(p, grid, st);
     }
     return cudaErrorInvalidValue;
 }

@@ -71,19 +71,20 @@ cudaError_t B2F_CAT(b2f_launch_kb_part, B2F_PART)(int R, int mode, const KBParam
     return cudaErrorInvalidValue;
 }
 
-// the same row lengths for the [pair][row][2] block layout of the round-2 column kernel
+// the same row lengths for the [pair][row][2] block layout of the round-2 column kernel; R = 256 uses the tile row pass
+// (b2f_kt.cu) instead
+#if B2F_PART != 2
 cudaError_t B2F_CAT(b2f_launch_kr_part, B2F_PART)(int R, int mode, const KBParams& p, int grid, cudaStream_t st) {
     switch (R) {
 #if B2F_PART == 0
         case 16: return by_mode_r<4, 4>(mode, p, grid, st);
         case 32: return by_mode_r<4, 8>(mode, p, grid, st);
         case 64: return by_mode_r<8, 8>(mode, p, grid, st);
-#elif B2F_PART == 1
+#else
         case 128: return by_mode_r<8, 16>(mode, p, grid, st);
         case 512: return by_mode_r<16, 32>(mode, p, grid, st);
-#else
-        case 256: return by_mode_r<16, 16>(mode, p, grid, st);
 #endif
     }
     return cudaErrorInvalidValue;
 }
+#endif

@@ -140,6 +140,7 @@ __device__ __forceinline__ uint4 expand_word_1bit(uint32_t w, bool masked) {
 
 constexpr int kK0Threads = 256;
 constexpr int kK0Stages = 4;
+constexpr int kK0CtasPerSM = 4;
 
 template <bool VEC>
 __global__ void __launch_bounds__(kK0Threads) k0_validate_compact(const K0Params p) {
@@ -647,9 +648,6 @@ struct KAParams {
     int R, nstrips, nblk, nif, payload_bytes, groups_per_slot;
     int64_t gb_begin, gb_end;   // this launch covers FFT blocks [gb_begin, gb_end); inter is indexed gb - gb_begin
     int64_t blk_step_bytes;     // stream bytes between the starts of consecutive blocks (= block size unless overlap-save)
-    int* sm_slots;           // [>= #SMs] arrival counters used to stagger co-resident CTAs
-    int stagger_cycles;
-    int variant;             // 0 = product kernel; else a timing ablation
     float in8_offset;        // 8-bit samples: value = code - in8_offset (127.5, or 128: SURVEY D3)
     const float4* levels; int64_t levels_stride;   // NBIT 22 (JA98): levels per window of 512 stream samples and IF (kj_levels_stream)
 };
@@ -665,16 +663,11 @@ struct KASmem {
 
 // R (row length = 2*nchan) is a template parameter so that every global and shared address
 // in the loop body is base + immediate.
-// VAR != 0 are timing ablations (wrong results, used by tools/ablate.py only): bit 0 drops the
-// butterflies, bit 1 the table twiddles, bit 2 the shared-memory exchanges.
-template <int NBIT, int R, int VAR = 0>
+// FWD_ONLY: forward transform only.  The kernel stops after A'[k2][n1] = FFT_512(column) * W_M^(k2 n1)
+// and stores it; used by the dedispersion path, where the chirp has to be applied between the row FFT
+// and the backward FFT.
+template <int NBIT, int R, bool FWD_ONLY>
 __global__ void __launch_bounds__(kKAThreads, kKACtasPerSM) ka_column_pass(const KAParams p) {
-    constexpr bool kFFT = !(VAR & 1), kTW = !(VAR & 2), kXCH = !(VAR & 4);
-    constexpr bool kOneBlock = (VAR & 8) != 0, kNoStore = (VAR & 16) != 0;   // bit 3: all stores hit block 0; bit 4: none
-    // bit 5 is a product mode, not an ablation: forward transform only.  The kernel stops after
-    // A'[k2][n1] = FFT_512(column) * W_M^(k2 n1) and stores it; used by the dedispersion path, where
-    // the chirp has to be applied between the row FFT and the backward FFT.
-    constexpr bool kFwdOnly = (VAR & 32) != 0;
     using S = KASmem<NBIT>;
     extern __shared__ __align__(16) uint8_t ka_smem[];
     float2* data = reinterpret_cast<float2*>(ka_smem);      // 512 points x 16 lanes, as [256 pairs][16] float4
@@ -715,23 +708,6 @@ __global__ void __launch_bounds__(kKAThreads, kKACtasPerSM) ka_column_pass(const
         const float m0 = (c0 == 0 || c0 == 3) ? kLevHi : kLevLo;
         const float m1 = (c1 == 0 || c1 == 3) ? kLevHi : kLevLo;
         s_lut[tid] = tid < 16 ? make_float2((c0 & 2) ? m0 : -m0, (c1 & 2) ? m1 : -m1) : make_float2(0.f, 0.f);
-    }
-
-    // Co-resident CTAs do identical work; started together they stay in lockstep and their
-    // shared-memory bursts collide.  Every second CTA to arrive on an SM waits half a work item
-    // once, so that one CTA's exchanges hide under the other's butterflies.
-    if (p.stagger_cycles > 0) {
-        __shared__ int s_slot;
-        if (tid == 0) {
-            unsigned smid;
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            s_slot = atomicAdd(&p.sm_slots[smid], 1) & 1;
-        }
-        __syncthreads();
-        if (s_slot) {
-            const long long t0 = clock64();
-            while (clock64() - t0 < p.stagger_cycles) {}
-        }
     }
 
     // P3's merged twiddle base for m1 = item: beta = W_M^(n1) * conj(W_512^(item))
@@ -792,7 +768,6 @@ __global__ void __launch_bounds__(kKAThreads, kKACtasPerSM) ka_column_pass(const
         // so every exchange is one 128-bit access per two points (the LSU instruction queue, not
         // bandwidth, was the limiter with 64-bit accesses).
         // ---- P1: decode + 16-point FFT over r (n2 = 32 r + l) for l = item and item+16, twiddle W_512^(l q)
-        float2 keepA[16], keepB[16];     // only live in the no-exchange ablation
         {
             float2 vA[16], vB[16];
 #pragma unroll
@@ -836,27 +811,22 @@ __global__ void __launch_bounds__(kKAThreads, kKACtasPerSM) ka_column_pass(const
                     }
                 }
             }
-            if (kFFT) { fft_inreg<16, false>(vA); fft_inreg<16, false>(vB); }
+            fft_inreg<16, false>(vA); fft_inreg<16, false>(vB);
             // (measured: computing these and the h^p powers in registers as well costs more FP than the
             //  32 table reads it saves -- 99.6 vs 96.8 ms/step -- so they stay in shared memory)
             const float4* twA = reinterpret_cast<const float4*>(s_w + item * 16);
             const float4* twB = reinterpret_cast<const float4*>(s_w + (item + 16) * 16);
 #pragma unroll
-            for (int q = 0; q < (kTW ? 16 : 0); q += 2) {
+            for (int q = 0; q < 16; q += 2) {
                 const float4 ta = twA[q >> 1], tb = twB[q >> 1];
                 if (q) vA[q] = cmul(vA[q], make_float2(ta.x, ta.y));
                 vA[q + 1] = cmul(vA[q + 1], make_float2(ta.z, ta.w));
                 if (q) vB[q] = cmul(vB[q], make_float2(tb.x, tb.y));
                 vB[q + 1] = cmul(vB[q + 1], make_float2(tb.z, tb.w));
             }
-            if (kXCH) {
 #pragma unroll
-                for (int q = 0; q < 16; ++q)
-                    data4[(q * 16 + item) * C + lane16] = make_float4(vA[q].x, vA[q].y, vB[q].x, vB[q].y);
-            } else {
-#pragma unroll
-                for (int q = 0; q < 16; ++q) { keepA[q] = vA[q]; keepB[q] = vB[q]; }
-            }
+            for (int q = 0; q < 16; ++q)
+                data4[(q * 16 + item) * C + lane16] = make_float4(vA[q].x, vA[q].y, vB[q].x, vB[q].y);
         }
         __syncthreads();
 
@@ -866,17 +836,12 @@ __global__ void __launch_bounds__(kKAThreads, kKACtasPerSM) ka_column_pass(const
             float2 u[32];
 #pragma unroll
             for (int l = 0; l < 16; ++l) {
-                if (kXCH) {
-                    const float4 t = data4[(q * 16 + l) * C + lane16];
-                    u[l] = make_float2(t.x, t.y);
-                    u[l + 16] = make_float2(t.z, t.w);
-                } else {
-                    u[l] = keepA[l];
-                    u[l + 16] = keepB[l];
-                }
+                const float4 t = data4[(q * 16 + l) * C + lane16];
+                u[l] = make_float2(t.x, t.y);
+                u[l + 16] = make_float2(t.z, t.w);
             }
-            if (kFFT) fft_inreg<32, false>(u);
-            if (kFwdOnly) {
+            fft_inreg<32, false>(u);
+            if (FWD_ONLY) {
                 // u[pp] = A[k2 = q + 16 pp]; full twiddle W_M^(k2 n1) = h^pp g^q, then straight to global
                 const float4 g4 = s_g4[(q & 7) * C + lane16];
                 const float2 gq = (q & 8) ? make_float2(g4.z, g4.w) : make_float2(g4.x, g4.y);
@@ -890,33 +855,28 @@ __global__ void __launch_bounds__(kKAThreads, kKACtasPerSM) ka_column_pass(const
             } else {
             if (q == 0) p.colsum[gb * R + n1] = u[0];          // A[k2 = 0]: column sum
 #pragma unroll
-            for (int pp = 0; pp < (kTW ? 16 : 0); ++pp) {
+            for (int pp = 0; pp < 16; ++pp) {
                 const float4 h = s_h4[pp * C + lane16];
                 if (pp) u[pp] = cmul(u[pp], make_float2(h.x, h.y));
                 u[pp + 16] = cmul(u[pp + 16], make_float2(h.z, h.w));
             }
-            if (kFFT) fft_inreg<32, true>(u);
+            fft_inreg<32, true>(u);
             // (the conj W_512^(q m1) twiddle of this stage is applied in P3, merged with W_M^(q n1))
-            if (kXCH) {
 #pragma unroll
-                for (int m = 0; m < 16; ++m)
-                    data4[(q * 16 + m) * C + lane16] = make_float4(u[m].x, u[m].y, u[m + 16].x, u[m + 16].y);
-            } else {
-#pragma unroll
-                for (int m = 0; m < 16; ++m) { keepA[m] = u[m]; keepB[m] = u[m + 16]; }
-            }
-            }   // !kFwdOnly
+            for (int m = 0; m < 16; ++m)
+                data4[(q * 16 + m) * C + lane16] = make_float4(u[m].x, u[m].y, u[m + 16].x, u[m + 16].y);
+            }   // !FWD_ONLY
         }
         __syncthreads();
-        if (kFwdOnly) continue;
+        if (FWD_ONLY) continue;
 
         // ---- P3: * W_M^(q n1) ; IFFT_16 over q -> m2 ; m = m1 + 32 m2 for m1 = item and item+16
         // twiddle of element q: W_M^(q n1) conj W_512^(q m1) = beta^q, beta = g conj(W_512^m1).
         // Round B has m1 + 16: beta_B^q = beta_A^q conj(W_32^q), a compile-time constant factor.
         {
             float2 pw[16];
-            if (kTW) cpowers15(betaS, pw);
-            float2* dA = p.inter + ((kOneBlock ? 0 : (gb - p.gb_begin)) * (int64_t)kL + item) * R + n1;
+            cpowers15(betaS, pw);
+            float2* dA = p.inter + ((gb - p.gb_begin) * (int64_t)kL + item) * R + n1;
             float2* dB = dA + 16 * R;
 #if B2F_P3_SPLIT
             // Round A is finished and stored before round B is even loaded (volatile accesses keep the assembler
@@ -926,52 +886,41 @@ __global__ void __launch_bounds__(kKAThreads, kKACtasPerSM) ka_column_pass(const
             float2 yA[16], yB[16];
 #pragma unroll
             for (int q = 0; q < 16; ++q) yA[q] = lds_v2_volatile(&data4[(q * 16 + item) * C + lane16]);
-            if (kTW) {
 #pragma unroll
-                for (int q = 1; q < 16; ++q) yA[q] = cmul(yA[q], pw[q]);
-            }
-            if (kFFT) fft_inreg<16, true>(yA);
+            for (int q = 1; q < 16; ++q) yA[q] = cmul(yA[q], pw[q]);
+            fft_inreg<16, true>(yA);
 #pragma unroll
             for (int m2 = 0; m2 < 16; ++m2) stg_v2_volatile(&dA[32 * m2 * R], yA[m2]);
 #pragma unroll
             for (int q = 0; q < 16; ++q)
                 yB[q] = lds_v2_volatile(reinterpret_cast<const float2*>(&data4[(q * 16 + item) * C + lane16]) + 1);
-            if (kTW) {
 #pragma unroll
-                for (int q = 1; q < 16; ++q) {
-                    const float2 cb = make_float2(cos64(2 * q), sin64(2 * q));
-                    yB[q] = cmul(cmul(yB[q], cb), pw[q]);
-                }
+            for (int q = 1; q < 16; ++q) {
+                const float2 cb = make_float2(cos64(2 * q), sin64(2 * q));
+                yB[q] = cmul(cmul(yB[q], cb), pw[q]);
             }
-            if (kFFT) fft_inreg<16, true>(yB);
+            fft_inreg<16, true>(yB);
 #pragma unroll
             for (int m2 = 0; m2 < 16; ++m2) dB[32 * m2 * R] = yB[m2];
 #else
             float2 yA[16], yB[16];
 #pragma unroll
             for (int q = 0; q < 16; ++q) {
-                if (kXCH) {
-                    const float4 t = data4[(q * 16 + item) * C + lane16];
-                    yA[q] = make_float2(t.x, t.y);
-                    yB[q] = make_float2(t.z, t.w);
-                } else {
-                    yA[q] = keepA[q];
-                    yB[q] = keepB[q];
-                }
+                const float4 t = data4[(q * 16 + item) * C + lane16];
+                yA[q] = make_float2(t.x, t.y);
+                yB[q] = make_float2(t.z, t.w);
             }
-            if (kTW) {
 #pragma unroll
-                for (int q = 1; q < 16; ++q) {
-                    yA[q] = cmul(yA[q], pw[q]);
-                    const float2 cb = make_float2(cos64(2 * q), sin64(2 * q));      // conj(W_32^q) = exp(+2 pi i q/32)
-                    yB[q] = cmul(cmul(yB[q], cb), pw[q]);
-                }
+            for (int q = 1; q < 16; ++q) {
+                yA[q] = cmul(yA[q], pw[q]);
+                const float2 cb = make_float2(cos64(2 * q), sin64(2 * q));      // conj(W_32^q) = exp(+2 pi i q/32)
+                yB[q] = cmul(cmul(yB[q], cb), pw[q]);
             }
-            if (kFFT) { fft_inreg<16, true>(yA); fft_inreg<16, true>(yB); }
+            fft_inreg<16, true>(yA); fft_inreg<16, true>(yB);
 #pragma unroll
             for (int m2 = 0; m2 < 16; ++m2) {
-                if (!kNoStore || yA[m2].x == 123456.789f) dA[32 * m2 * R] = yA[m2];
-                if (!kNoStore || yB[m2].x == 123456.789f) dB[32 * m2 * R] = yB[m2];
+                dA[32 * m2 * R] = yA[m2];
+                dB[32 * m2 * R] = yB[m2];
             }
 #endif
         }

@@ -3,16 +3,16 @@
 #pragma once
 #include "b2f_kernels.cuh"
 
-cudaError_t b2f_launch_ka(int in_nbit, int R, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
-cudaError_t b2f_launch_ka_22(int R, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
+// fwd_only: the column pass stops after the forward transform (dedispersion path)
+cudaError_t b2f_launch_ka(int in_nbit, int R, bool fwd_only, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
+cudaError_t b2f_launch_ka_22(int R, bool fwd_only, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
 cudaError_t b2f_launch_kb(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);
-cudaError_t b2f_launch_kr(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);     // [pair][row][2] blocks
+cudaError_t b2f_launch_kr(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);     // [pair][row][2] blocks, R != 256
 cudaError_t b2f_launch_kr_part0(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);
 cudaError_t b2f_launch_kr_part1(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);
-cudaError_t b2f_launch_kr_part2(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);
 cudaError_t b2f_launch_kc(int R, const b2f::KCParams& p, int grid, cudaStream_t st);
-cudaError_t b2f_launch_ka_2(int R, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
-cudaError_t b2f_launch_ka_8(int R, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
+cudaError_t b2f_launch_ka_2(int R, bool fwd_only, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
+cudaError_t b2f_launch_ka_8(int R, bool fwd_only, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
 cudaError_t b2f_launch_kb_part0(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);   // R = 16, 32, 64
 cudaError_t b2f_launch_kb_part1(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);   // R = 128, 512
 cudaError_t b2f_launch_kb_part2(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);   // R = 256
