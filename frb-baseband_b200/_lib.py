@@ -6,6 +6,7 @@ import ctypes as C
 import os
 
 B2F_MAX_IF = 32
+B2F_MAX_DM = 64
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("B2F_LIB") or os.path.join(_HERE, "libb2f.so")   # B2F_LIB: an alternative build (A/B kernel experiments)
 
@@ -33,6 +34,7 @@ class Params(C.Structure):
         ("decode_mode", C.c_int32), ("in8_offset_mode", C.c_int32), ("fft_normalised", C.c_int32),
         ("rescale_mode", C.c_int32), ("digi_sigma", C.c_double),
         ("raw_format", C.c_int32), ("reserved0", C.c_int32),
+        ("ndm", C.c_int32), ("dm_trials", C.c_double * B2F_MAX_DM),
     ]
 
 
@@ -42,6 +44,7 @@ class Geometry(C.Structure):
         ("chunk_rows", C.c_int64), ("block_samples", C.c_int64), ("samples_per_frame", C.c_int64),
         ("row_bytes", C.c_int64), ("nprod", C.c_int32), ("freq_res", C.c_int32), ("tsamp_s", C.c_double),
         ("interval_rows", C.c_int64), ("nfilt_pos", C.c_int32), ("nfilt_neg", C.c_int32),
+        ("ndm", C.c_int32), ("trial_row_bytes", C.c_int64),
     ]
 
 
@@ -71,7 +74,7 @@ class ScanIO(C.Structure):
         ("rawdatafile", C.c_char_p), ("telescope_id", C.c_int32), ("machine_id", C.c_int32),
         ("src_raj", C.c_double), ("src_dej", C.c_double), ("refdm", C.c_double), ("write_refdm", C.c_int32),
         ("ring", C.c_int32), ("readers_per_file", C.c_int32), ("part_index", C.c_int32), ("part_count", C.c_int32),
-        ("stats_only", C.c_int32),
+        ("stats_only", C.c_int32), ("trial_out_paths", C.POINTER(C.c_char_p)),
     ]
 
 

@@ -59,6 +59,9 @@ struct b2f_plan {
     int64_t interval_rows = 0, F_cap_rows = 0;
     int out_elem_bits = 8;
     int64_t row_elems = 0, row_bytes = 0;
+    // trial DMs (b2f_params.ndm): F, d_Fk, statistics and chirp tables hold ndm * nif slots, trial-major; 1 without trials
+    int ndm = 1;
+    int64_t trial_row_elems = 0;
 
     cudaStream_t stream = nullptr, copy_stream = nullptr, d2h_stream = nullptr;
     bool own_stream = false;
@@ -345,14 +348,14 @@ int init_state(b2f_plan* pl) {
     const int ncol = pl->nprod * pl->N;
     CU(cudaMemsetAsync(pl->d_counters, 0, C_COUNT * sizeof(unsigned long long), pl->stream));
     if (!pl->preset_stats) {
-        CU(cudaMemsetAsync(pl->d_mean, 0, (size_t)pl->prm.nif * ncol * sizeof(float), pl->stream));
+        CU(cudaMemsetAsync(pl->d_mean, 0, (size_t)pl->ndm * pl->prm.nif * ncol * sizeof(float), pl->stream));
         // keep_bandpass with normalised transforms (D4): the "scale" the digitiser applies is 1 / (M * freq_res), squared for -d3
         float unit = 1.0f;
         if (pl->prm.keep_bandpass && pl->prm.fft_normalised) {
             const double nrm = 1.0 / ((double)pl->M * pl->L);
             unit = (float)(pl->prm.pol_mode == B2F_POL_I2 ? nrm * nrm : nrm);
         }
-        std::vector<float> ones((size_t)pl->prm.nif * ncol, unit);
+        std::vector<float> ones((size_t)pl->ndm * pl->prm.nif * ncol, unit);
         CU(cudaMemcpyAsync(pl->d_scale, ones.data(), ones.size() * sizeof(float), cudaMemcpyHostToDevice, pl->stream));
     }
     CU(cudaStreamSynchronize(pl->stream));
@@ -478,10 +481,15 @@ int push_dedisp(b2f_plan* pl, int64_t nblk, int64_t T) {
             if (pl->dedisp) {
                 kx.gb_begin = b0; kx.gb_end = b0 + nb;
                 const int64_t work = nb * (pl->N / kx.CH);
-                rc = timed(pl, B2F_K_DEDISP, [&] {
-                    kx_dedisp_generic<<<(unsigned)std::min<int64_t>(work, (int64_t)pl->num_sms), kKXThreads, smem_kx, pl->stream>>>(kx);
-                });
-                if (rc) return rc;
+                for (int t = 0; t < pl->ndm; ++t) {             // trial DMs: the same channel samples, each trial's chirp and F slots
+                    KXParams kt = kx;
+                    kt.chirp = kx.chirp + (int64_t)t * nif * pl->L * pl->N;
+                    kt.F = kx.F + (int64_t)t * nif * kx.F_if_stride;
+                    rc = timed(pl, B2F_K_DEDISP, [&] {
+                        kx_dedisp_generic<<<(unsigned)std::min<int64_t>(work, (int64_t)pl->num_sms), kKXThreads, smem_kx, pl->stream>>>(kt);
+                    });
+                    if (rc) return rc;
+                }
             }
         }
     } else if (nblk > 0) {
@@ -505,7 +513,8 @@ int push_dedisp(b2f_plan* pl, int64_t nblk, int64_t T) {
         kc.spec = pl->d_spec; kc.chirp = pl->d_chirp; kc.tab_w = pl->d_tab_w;
         kc.F = row_dst(pl); kc.F_if_stride = row_dst_stride(pl); kc.row0 = row_dst_row0(pl);
         kc.nblk = (int)nblk; kc.nif = nif; kc.D = pl->D; kc.mode = pl->prm.pol_mode;
-        kc.nfilt_pos = pl->nfilt_pos; kc.keep = pl->keep;
+        kc.nfilt_pos = pl->nfilt_pos; kc.keep = pl->keep; kc.ndm = pl->ndm;
+        const bool trials = pl->prm.ndm > 0;            // kc_dedisp_trials: one CTA per SM (registers hold the un-mixed spectrum)
         int TR, PT;
         kb_shape(pl->R, &TR, &PT);
         const int RW = 32 / TR;
@@ -525,7 +534,9 @@ int push_dedisp(b2f_plan* pl, int64_t nblk, int64_t T) {
             if (e != cudaSuccess) return fail(B2F_ECUDA, std::string("row pass launch: ") + cudaGetErrorString(e));
             kc.gb_begin = b0; kc.gb_end = b0 + nb;
             const int64_t work = nb * (pl->N / 8);
-            rc = timed(pl, B2F_K_DEDISP, [&] { e = b2f_launch_kc(pl->R, kc, (int)std::min<int64_t>(work, (int64_t)pl->num_sms * 2), pl->stream); });
+            rc = timed(pl, B2F_K_DEDISP, [&] {
+                e = b2f_launch_kc(pl->R, kc, trials, (int)std::min<int64_t>(work, (int64_t)pl->num_sms * (trials ? 1 : 2)), pl->stream);
+            });
             if (rc) return rc;
             if (e != cudaSuccess) return fail(B2F_ECUDA, std::string("dedispersion back end launch: ") + cudaGetErrorString(e));
         }
@@ -752,7 +763,7 @@ static __global__ void kd_sum_rows(const float* __restrict__ Fk, int64_t Fk_if_s
 namespace {
 int sum_rows(b2f_plan* pl, int64_t krows, int64_t rows) {
     if (pl->tsq <= 1) return 0;
-    const int ncol = pl->nprod * pl->N, nif = pl->prm.nif;
+    const int ncol = pl->nprod * pl->N, nif = pl->ndm * pl->prm.nif;     // every (trial, IF) slot
     const int64_t total = pl->fk_pending + krows, left = total - rows * pl->tsq;
     if (rows > 0) {
         const int64_t n = rows * ncol;
@@ -796,10 +807,24 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
         return fail(B2F_EINVAL, "nbit not in supported values of [2, 8, 16, -32]");
     if (!(prm->in_nbit == 1 || prm->in_nbit == 2 || prm->in_nbit == 8)) return fail(B2F_EUNSUPPORTED, "VDIF bits/sample must be 1, 2 or 8");
     if (prm->nchan < 1) return fail(B2F_EINVAL, "nchan");
+    // trial DMs: one coherent plan writes ndm filterbanks; its geometry is that of a single-DM plan at the largest trial
+    if (prm->ndm < 0 || prm->ndm > B2F_MAX_DM) return fail(B2F_EINVAL, "ndm must be 0..64 (B2F_MAX_DM)");
+    double dm = prm->dm;
+    if (prm->ndm > 0) {
+        if (prm->coherent != 1) return fail(B2F_EINVAL, "trial DMs need coherent = 1");
+        if (prm->dm != 0.0) return fail(B2F_EINVAL, "trial DMs are given in dm_trials: dm must be 0");
+        for (int k = 0; k < prm->ndm; ++k) {
+            const double t = prm->dm_trials[k];
+            if (!std::isfinite(t) || t < 0) return fail(B2F_EINVAL, "trial DMs must be finite and >= 0");
+            if (k > 0 && !(t > prm->dm_trials[k - 1])) return fail(B2F_EINVAL, "trial DMs must be strictly increasing");
+        }
+        dm = prm->dm_trials[prm->ndm - 1];
+        if (!(dm > 0)) return fail(B2F_EINVAL, "the largest trial DM must be > 0");
+    }
     int L = prm->freq_res > 0 ? prm->freq_res : (prm->nchan <= 128 ? 512 : 2 * prm->nchan);
     const int R = 2 * prm->nchan;
     if (!is_pow2(R) || R < 16 || R > 8192) return fail(B2F_EUNSUPPORTED, "nchan must be a power of two in 8..4096");
-    const bool dedisp = prm->coherent && prm->dm > 0.0;
+    const bool dedisp = prm->coherent && dm > 0.0;
     // overlap-save samples discarded at each end of a block and channel: half the smearing across the lowest channel of
     // the lowest subband (8.3 us DM dnu/nu_GHz^3, the rule of submit_job.py:62) plus 10 %, rounded up to a multiple of the
     // integration factor so that every block yields whole output samples
@@ -807,7 +832,7 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
         const double bw0 = std::fabs(prm->bw_mhz[0]);
         double fmin = 1e30;
         for (int i = 0; i < prm->nif; ++i) fmin = std::min(fmin, prm->freq_mhz[i] - bw0 / 2 + bw0 / prm->nchan / 2);
-        const double ns = 8.3 * prm->dm * (bw0 / prm->nchan) / std::pow(fmin / 1000.0, 3) / ((double)prm->nchan / bw0);
+        const double ns = 8.3 * dm * (bw0 / prm->nchan) / std::pow(fmin / 1000.0, 3) / ((double)prm->nchan / bw0);
         int nf = (int)std::ceil(0.55 * ns);
         nf = (nf + Dint - 1) / Dint * Dint;
         return nf < Dint ? Dint : nf;
@@ -831,7 +856,7 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     if (D_user > (1 << 20)) return fail(B2F_EUNSUPPORTED, "tscrunch above 2^20");
     int D = D_user & -D_user;                       // what the kernels integrate; kd_sum_rows adds tsq = D_user / D of their rows
     while (D > L) D >>= 1;
-    if (prm->coherent && prm->dm > 0.0) while (D > 128) D >>= 1;
+    if (dedisp) while (D > 128) D >>= 1;
     const int tsq = D_user / D;
     if (prm->header_bytes != 32 && prm->header_bytes != 16) return fail(B2F_EINVAL, "header_bytes must be 32 or 16");
     const int payload = prm->frame_bytes - prm->header_bytes;
@@ -935,7 +960,9 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     pl->interval_rows = prm->keep_bandpass ? 0 : (int64_t)llround(interval / tsamp);
     pl->F_cap_rows = pl->interval_rows + 2 * pl->chunk_rows;
     pl->out_elem_bits = prm->out_nbit == -32 ? 32 : prm->out_nbit;
-    pl->row_elems = (int64_t)prm->nif * nprod * prm->nchan;
+    pl->ndm = std::max(1, prm->ndm);
+    pl->trial_row_elems = (int64_t)prm->nif * nprod * prm->nchan;
+    pl->row_elems = pl->ndm * pl->trial_row_elems;
     pl->row_bytes = pl->row_elems * pl->out_elem_bits / 8;
     {
         // FFT blocks per column/row launch pair.  0 = the whole push.  L2-sized sub-batches (e.g. 72
@@ -1016,6 +1043,24 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     }
     const int nif = prm->nif;
     const int64_t nbt = (int64_t)nif * pl->chunk_blocks;
+    const int nslot = pl->ndm * nif;                        // F / statistics slots: (trial, IF), trial-major
+    pl->F_if_stride = pl->F_cap_rows * nprod * pl->N;
+    if (tsq > 1) pl->Fk_if_stride = (pl->chunk_blocks * pl->keep / D + tsq) * nprod * pl->N;
+    if (prm->ndm > 0) {
+        // what grows with the trials, and the two spectrum-sized buffers, against what the device has free
+        const int64_t blocks = pl->batch_blocks > 0 ? std::min<int64_t>(pl->batch_blocks, nbt) : nbt;
+        const double need = (double)nslot * ((pl->F_if_stride + pl->Fk_if_stride) * sizeof(float) +
+                                             (double)nprod * pl->N * (kStatSplit * sizeof(double2) + 2 * sizeof(float)) +
+                                             (double)L * pl->N * sizeof(float2)) +
+                            2.0 * blocks * L * R * sizeof(float2);
+        size_t fr = 0, tot = 0;
+        CUB(cudaMemGetInfo(&fr, &tot));
+        if (need > (double)fr) {
+            g_err = "ndm = " + std::to_string(prm->ndm) + " trial DMs need " + std::to_string((int64_t)(need / (1 << 20))) + " MiB of device memory, " +
+                    std::to_string((int64_t)(fr >> 20)) + " MiB are free: use fewer trials or a smaller chunk_units";
+            return bail(B2F_ENOMEM);
+        }
+    }
     pl->slot_bytes = W ? (int)spf : (prm->in_nbit == 8 ? payload : (int)spf);         // 1- and 2-bit: one index byte per time sample
     pl->compact_stride = (size_t)((pl->chunk_frames * (int64_t)pl->slot_bytes + (pl->carry_mode ? pl->M * pl->bps : 0) + 255) / 256 * 256);
     pl->wmask_stride = (size_t)((pl->chunk_frames * pl->groups_per_slot + (pl->smask ? pl->M * pl->bps / 32 : 0) + 255) / 256 * 256);
@@ -1047,15 +1092,11 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     CUB(cudaMalloc(&pl->d_inter, (size_t)inter_blocks * L * R * sizeof(float2)));
     CUB(cudaMalloc(&pl->d_colsum, (size_t)nbt * R * sizeof(float2)));
     CUB(cudaMalloc(&pl->d_eps, (size_t)nbt * pl->N * sizeof(float2)));
-    pl->F_if_stride = pl->F_cap_rows * nprod * pl->N;
-    CUB(cudaMalloc(&pl->d_F, (size_t)pl->F_if_stride * nif * sizeof(float)));
-    if (tsq > 1) {
-        pl->Fk_if_stride = (pl->chunk_blocks * pl->keep / D + tsq) * nprod * pl->N;
-        CUB(cudaMalloc(&pl->d_Fk, (size_t)pl->Fk_if_stride * nif * sizeof(float)));
-    }
-    CUB(cudaMalloc(&pl->d_mean, (size_t)nif * nprod * pl->N * sizeof(float)));
-    CUB(cudaMalloc(&pl->d_scale, (size_t)nif * nprod * pl->N * sizeof(float)));
-    CUB(cudaMalloc(&pl->d_partial, (size_t)nif * kStatSplit * nprod * pl->N * sizeof(double2)));
+    CUB(cudaMalloc(&pl->d_F, (size_t)pl->F_if_stride * nslot * sizeof(float)));
+    if (tsq > 1) CUB(cudaMalloc(&pl->d_Fk, (size_t)pl->Fk_if_stride * nslot * sizeof(float)));
+    CUB(cudaMalloc(&pl->d_mean, (size_t)nslot * nprod * pl->N * sizeof(float)));
+    CUB(cudaMalloc(&pl->d_scale, (size_t)nslot * nprod * pl->N * sizeof(float)));
+    CUB(cudaMalloc(&pl->d_partial, (size_t)nslot * kStatSplit * nprod * pl->N * sizeof(double2)));
     CUB(cudaMalloc(&pl->d_counters, C_COUNT * sizeof(unsigned long long)));
     if (pl->carry_mode) CUB(cudaMalloc(&pl->d_carry, (size_t)pl->M * pl->bps * nif));
     if (pl->smask) CUB(cudaMalloc(&pl->d_carry_mask, (size_t)pl->M * pl->bps / 32 * nif));
@@ -1102,17 +1143,20 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     }
     if (dedisp) {
         CUB(cudaMalloc(&pl->d_spec, (size_t)inter_blocks * L * R * sizeof(float2)));
-        // chirp H[if][k2][c] = exp(-i 2 pi D DM 1e6 f^2 / (fc^2 (fc + f))), conjugated for LSB, in double
-        std::vector<float2> h((size_t)nif * L * prm->nchan);
-        for (int i = 0; i < nif; ++i) {
-            const double bw = prm->bw_mhz[i], chbw = bw / prm->nchan;
-            for (int c = 0; c < prm->nchan; ++c) {
-                const double fc = prm->freq_mhz[i] - bw / 2 + (c + 0.5) * chbw;
-                for (int k2 = 0; k2 < L; ++k2) {
-                    const double f = ((double)k2 / L - 0.5) * chbw;
-                    double ph = 2.0 * M_PI * (1.0 / 2.41e-4) * 1e6 * prm->dm * f * f / (fc * fc * (fc + f));
-                    if (bw < 0) ph = -ph;
-                    h[((size_t)i * L + k2) * prm->nchan + c] = make_float2((float)cos(ph), (float)-sin(ph));
+        // chirp H[trial][if][k2][c] = exp(-i 2 pi D DM 1e6 f^2 / (fc^2 (fc + f))), conjugated for LSB, in double
+        std::vector<float2> h((size_t)nslot * L * prm->nchan);
+        for (int t = 0; t < pl->ndm; ++t) {
+            const double dmt = prm->ndm > 0 ? prm->dm_trials[t] : prm->dm;
+            for (int i = 0; i < nif; ++i) {
+                const double bw = prm->bw_mhz[i], chbw = bw / prm->nchan;
+                for (int c = 0; c < prm->nchan; ++c) {
+                    const double fc = prm->freq_mhz[i] - bw / 2 + (c + 0.5) * chbw;
+                    for (int k2 = 0; k2 < L; ++k2) {
+                        const double f = ((double)k2 / L - 0.5) * chbw;
+                        double ph = 2.0 * M_PI * (1.0 / 2.41e-4) * 1e6 * dmt * f * f / (fc * fc * (fc + f));
+                        if (bw < 0) ph = -ph;
+                        h[(((size_t)t * nif + i) * L + k2) * prm->nchan + c] = make_float2((float)cos(ph), (float)-sin(ph));
+                    }
                 }
             }
         }
@@ -1149,6 +1193,8 @@ int b2f_get_geometry(const b2f_plan* pl, b2f_geometry* g) {
     g->interval_rows = pl->interval_rows;
     g->nfilt_pos = pl->nfilt_pos;
     g->nfilt_neg = pl->nfilt_neg;
+    g->ndm = pl->ndm;
+    g->trial_row_bytes = pl->trial_row_elems * pl->out_elem_bits / 8;
     return 0;
 }
 
@@ -1176,7 +1222,7 @@ int b2f_push(b2f_plan* pl, const void* const* frames, int64_t nframes, int on_de
         // running rescale keeps the rows of an unfinished interval: move them to the front of the buffer, in pieces no
         // longer than the gap so that source and destination of one copy never overlap
         const int64_t ncolF = (int64_t)pl->nprod * pl->N;
-        for (int i = 0; i < pl->prm.nif; ++i)
+        for (int i = 0; i < pl->ndm * pl->prm.nif; ++i)
             for (int64_t r0 = 0; r0 < pl->rows_held; r0 += pl->rows_off) {
                 const int64_t n = std::min(pl->rows_off, pl->rows_held - r0);
                 float* base = pl->d_F + i * pl->F_if_stride;
@@ -1392,6 +1438,7 @@ int b2f_pull(b2f_plan* pl, void* out, int64_t max_rows, int out_on_device, int64
 }
 
 int b2f_pull_strided(b2f_plan* pl, void* out, int64_t max_rows, int64_t row_pitch_bytes, int64_t* nrows) {
+    if (pl && pl->prm.ndm > 0) return fail(B2F_EUNSUPPORTED, "b2f_pull_strided splices the tiles of one DM: not with trial DMs");
     if (pl && row_pitch_bytes < pl->row_bytes) return fail(B2F_EINVAL, "row pitch smaller than one output row");
     {
         // kq_quantise stores 4 output elements at a time: 4 bytes for 8-bit (1 byte for 2-bit), 8 for 16-bit, 16 for float
@@ -1412,9 +1459,9 @@ static int pull_impl(b2f_plan* pl, void* out, int64_t max_rows, int out_on_devic
         if (pl->rows_held >= pl->interval_rows || (pl->flushed && pl->rows_held > 0)) {
             const int64_t nstat = std::min(pl->rows_held, pl->interval_rows);
             int rc = timed(pl, B2F_K_STATS, [&] {
-                dim3 g1((ncol + 127) / 128, nif, kStatSplit);
+                dim3 g1((ncol + 127) / 128, pl->ndm * nif, kStatSplit);
                 ks_partial<<<g1, 128, 0, pl->stream>>>(pl->d_F + pl->rows_off * ncol, pl->F_if_stride, nstat, ncol, pl->d_partial);
-                dim3 g2((ncol + 127) / 128, nif);
+                dim3 g2((ncol + 127) / 128, pl->ndm * nif);
                 ks_final<<<g2, 128, 0, pl->stream>>>(pl->d_partial, kStatSplit, nstat, ncol, pl->d_mean, pl->d_scale);
             });
             if (rc) return rc;
@@ -1452,6 +1499,7 @@ static int pull_impl(b2f_plan* pl, void* out, int64_t max_rows, int out_on_devic
     kq.nif = nif; kq.nprod = pl->nprod; kq.nchan = pl->N; kq.out_nbit = pl->prm.out_nbit;
     kq.pol_major = pl->prm.splice_pol_major;
     kq.inv_digi_sigma = (float)(1.0 / (pl->prm.digi_sigma > 0 ? pl->prm.digi_sigma : 6.0));
+    kq.trial_row_elems = (int)pl->trial_row_elems;
     for (int i = 0; i < nif; ++i) {
         kq.if_order[i] = pl->prm.if_order[i];
         kq.flip[i] = pl->prm.bw_mhz[i] > 0 ? 1 : 0;
@@ -1546,7 +1594,7 @@ int b2f_get_rescale(b2f_plan* pl, float* mean, float* scale) {
     if (!pl || !mean || !scale) return fail(B2F_EINVAL, "null argument");
     CU(cudaSetDevice(pl->prm.device));
     CU(cudaStreamSynchronize(pl->stream));
-    const size_t n = (size_t)pl->prm.nif * pl->nprod * pl->N * sizeof(float);
+    const size_t n = (size_t)pl->ndm * pl->prm.nif * pl->nprod * pl->N * sizeof(float);
     CU(cudaMemcpy(mean, pl->d_mean, n, cudaMemcpyDeviceToHost));
     CU(cudaMemcpy(scale, pl->d_scale, n, cudaMemcpyDeviceToHost));
     return 0;
@@ -1561,7 +1609,7 @@ int b2f_set_rescale(b2f_plan* pl, const float* mean, const float* scale) {
         pl->stats_ready = pl->prm.keep_bandpass != 0;
         return 0;
     }
-    const size_t n = (size_t)pl->prm.nif * pl->nprod * pl->N * sizeof(float);
+    const size_t n = (size_t)pl->ndm * pl->prm.nif * pl->nprod * pl->N * sizeof(float);
     CU(cudaStreamSynchronize(pl->stream));
     CU(cudaMemcpy(pl->d_mean, mean, n, cudaMemcpyHostToDevice));
     CU(cudaMemcpy(pl->d_scale, scale, n, cudaMemcpyHostToDevice));
@@ -1743,7 +1791,7 @@ int b2f_debug_copy(b2f_plan* pl, int which, void* dst, size_t nbytes, size_t* ne
         }
         case 5: src = pl->d_colsum; n = (size_t)nbt * pl->R * sizeof(float2); break;
         case 6: src = pl->d_eps; n = (size_t)nbt * pl->N * sizeof(float2); break;
-        case 7: src = pl->d_F; n = (size_t)pl->F_if_stride * nif * sizeof(float); break;
+        case 7: src = pl->d_F; n = (size_t)pl->F_if_stride * pl->ndm * nif * sizeof(float); break;
         case 8: src = pl->d_fprof; n = (size_t)pl->f_grid * kFWarps * 8 * sizeof(unsigned long long); break;
         default: return fail(B2F_EINVAL, "which");
     }

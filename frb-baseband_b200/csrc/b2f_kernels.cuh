@@ -1400,14 +1400,119 @@ __global__ void __launch_bounds__(kKBThreads, 2) kr_row_pass(const KBParams p) {
 // [nfilt_pos, 512 - nfilt_neg), detects (partner polarisation by shuffle) and integrates D samples.
 struct KCParams {
     const float2* spec;         // [gb - gb_begin][512][R]
-    const float2* chirp;        // [nif][512][N]  H[c][k2] stored k2-major
+    const float2* chirp;        // [ndm][nif][512][N]  H[c][k2] stored k2-major
     const float2* tab_w;        // [32][16] W_512^(l q)
-    float* F; int64_t F_if_stride; int64_t row0;
+    float* F; int64_t F_if_stride; int64_t row0;  // F slot of (trial t, IF i): t * nif + i
     int nblk, nif, D, mode, nfilt_pos, keep;      // keep = 512 - nfilt_pos - nfilt_neg (multiple of D)
     int64_t gb_begin, gb_end;
+    int ndm;                                      // trial DMs (kc_dedisp_trials); kc_dedisp_back runs trial 0
 };
 
 constexpr size_t kKCSmemBytes = (size_t)(kL * 16 + 512) * sizeof(float2);
+
+// (z1 + conj z2)/2 for pol 0, (z1 - conj z2)/(2i) for pol 1: the spectrum of one polarisation from the mixed block spectrum
+__device__ __forceinline__ float2 kc_unmix(float2 z1, float2 z2, int pol) {
+    float2 x;
+    if (pol == 0) x = make_float2(0.5f * (z1.x + z2.x), 0.5f * (z1.y - z2.y));
+    else          x = make_float2(0.5f * (z1.y + z2.y), -0.5f * (z1.x - z2.x));
+    return x;
+}
+
+// Spectrum bin k2 = 32 a + item + 16 h of channel c, and its mirror M - (c L + k2): row L - k2, channel R-1-c (k2 > 0) or
+// row 0, channel (R-c) mod R.
+template <int R>
+__device__ __forceinline__ float2 kc_load_unmixed(const float2* Z, int k2, int c, int pol) {
+    const float2 z1 = Z[(int64_t)k2 * R + c];
+    const float2 z2 = k2 ? Z[(int64_t)(kL - k2) * R + (R - 1 - c)] : Z[(R - c) & (R - 1)];
+    return kc_unmix(z1, z2, pol);
+}
+
+// Everything after the chirp for one (block, 8-channel strip): vA / vB hold the chirped bins k2 = 32 a + item (+ 16).
+// IFFT_16 over a, twiddle, exchange, IFFT_32 over l, detect into shared memory, integrate D kept samples per output row
+// into F slot `slot` (trial * nif + IF).  Ends with a barrier: the shared buffers are free again.
+template <int R>
+__device__ __forceinline__ void kc_backward_detect(float2 (&vA)[16], float2 (&vB)[16], const KCParams& p, float4* data4, float* pw,
+                                                   const float2* s_w, int nprod, bool own_only, int slot, int64_t blk, int strip) {
+    constexpr int N = R / 2;
+    const int tid = threadIdx.x, lane16 = tid & 15, item = tid >> 4;
+    const int ch8 = lane16 >> 1, pol = lane16 & 1;
+    {
+        fft_inreg<16, true>(vA);
+        fft_inreg<16, true>(vB);
+        const float4* twA = reinterpret_cast<const float4*>(s_w + item * 16);
+        const float4* twB = reinterpret_cast<const float4*>(s_w + (item + 16) * 16);
+#pragma unroll
+        for (int q = 0; q < 16; q += 2) {            // * conj W_512^(l m_lo)
+            const float4 ta = twA[q >> 1], tb = twB[q >> 1];
+            if (q) vA[q] = cmul_conj(vA[q], make_float2(ta.x, ta.y));
+            vA[q + 1] = cmul_conj(vA[q + 1], make_float2(ta.z, ta.w));
+            if (q) vB[q] = cmul_conj(vB[q], make_float2(tb.x, tb.y));
+            vB[q + 1] = cmul_conj(vB[q + 1], make_float2(tb.z, tb.w));
+        }
+#pragma unroll
+        for (int q = 0; q < 16; ++q)
+            data4[(q * 16 + item) * 16 + lane16] = make_float4(vA[q].x, vA[q].y, vB[q].x, vB[q].y);
+    }
+    __syncthreads();
+    // ---- P2: IFFT_32 over l for m_lo = item -> y[m = m_lo + 16 m_hi]; detect into smem
+    {
+        float2 u[32];
+#pragma unroll
+        for (int l = 0; l < 16; ++l) {
+            const float4 t = data4[(item * 16 + l) * 16 + lane16];
+            u[l] = make_float2(t.x, t.y);
+            u[l + 16] = make_float2(t.z, t.w);
+        }
+        fft_inreg<32, true>(u);
+        __syncthreads();                   // everyone has its u[]: the exchange buffer becomes the power buffer
+        if (own_only) {
+            // products without a cross term: every lane squares its own polarisation, [m][ch][pol]
+#pragma unroll
+            for (int mh = 0; mh < 32; ++mh)
+                pw[(size_t)(item + 16 * mh) * 16 + lane16] = u[mh].x * u[mh].x + u[mh].y * u[mh].y;
+        } else {
+#pragma unroll
+        for (int mh = 0; mh < 32; ++mh) {
+            const float ox = __shfl_xor_sync(0xffffffffu, u[mh].x, 1), oy = __shfl_xor_sync(0xffffffffu, u[mh].y, 1);
+            if (pol == 0) {                 // this lane holds yP, its neighbour yQ
+                const float2 yP = u[mh], yQ = make_float2(ox, oy);
+                const float pp = yP.x * yP.x + yP.y * yP.y, qq = yQ.x * yQ.x + yQ.y * yQ.y;
+                const float re = yP.x * yQ.x + yP.y * yQ.y, im = yP.y * yQ.x - yP.x * yQ.y;   // yP conj(yQ)
+                float* dst = pw + (size_t)(item + 16 * mh) * 8 + ch8;
+                constexpr size_t PS = (size_t)kL * 8;        // product stride
+                switch (p.mode) {
+                    case B2F_POL_I2: dst[0] = (pp + qq) * (pp + qq); break;
+                    case B2F_POL_COHERENCE: dst[0] = pp; dst[PS] = qq; dst[2 * PS] = re; dst[3 * PS] = im; break;
+                    default: dst[0] = pp + qq; dst[PS] = 2.f * re; dst[2 * PS] = 2.f * im; dst[3 * PS] = pp - qq; break;
+                }
+            }
+        }
+        }
+    }
+    __syncthreads();
+    // ---- integrate D kept samples per output row
+    const int nrow = p.keep / p.D;
+    const int64_t t0 = p.row0 + blk * nrow;
+    for (int o = tid; o < nprod * nrow * 8; o += 256) {
+        const int ch = o & 7, r = (o >> 3) % nrow, k = (o >> 3) / nrow;
+        float sum = 0.f;
+        if (own_only) {
+            const float2* src = reinterpret_cast<const float2*>(pw) + (size_t)(p.nfilt_pos + r * p.D) * 8 + ch;
+            float s0 = 0.f, s1 = 0.f;
+            for (int i = 0; i < p.D; ++i) {
+                const float2 v = src[i * 8];
+                s0 += v.x;
+                s1 += v.y;
+            }
+            sum = p.mode == B2F_POL_I ? s0 + s1 : p.mode == B2F_POL_P0 ? s0 : p.mode == B2F_POL_P1 ? s1 : (k == 0 ? s0 : s1);
+        } else {
+            const float* src = pw + ((size_t)k * kL + p.nfilt_pos + r * p.D) * 8 + ch;
+            for (int i = 0; i < p.D; ++i) sum += src[i * 8];
+        }
+        p.F[slot * p.F_if_stride + (t0 + r) * (int64_t)(nprod * N) + k * N + strip * 8 + ch] = sum;
+    }
+    __syncthreads();
+}
 
 template <int R>
 __global__ void __launch_bounds__(256, 2) kc_dedisp_back(const KCParams p) {
@@ -1527,6 +1632,54 @@ __global__ void __launch_bounds__(256, 2) kc_dedisp_back(const KCParams p) {
             p.F[ifi * p.F_if_stride + (t0 + r) * (int64_t)(nprod * N) + k * N + (int)(w % nstrips) * 8 + ch] = sum;
         }
         __syncthreads();
+    }
+}
+
+// Several trial DMs in one pass (b2f_params.ndm): per (block, 8-channel strip) the spectrum is loaded and un-mixed once and
+// kept in registers (64 per thread, hence one CTA of 256 threads per SM); then, for each trial, the same chirp multiply,
+// backward FFT, overlap discard, detection and integration as kc_dedisp_back, into that trial's F slots.  The arithmetic
+// per trial is kc_dedisp_back's, so every trial is bit-identical to a single-DM plan with the same nfilt.
+template <int R>
+__global__ void __launch_bounds__(256, 1) kc_dedisp_trials(const KCParams p) {
+    constexpr int N = R / 2;
+    extern __shared__ __align__(16) uint8_t kc_smem[];
+    float4* data4 = reinterpret_cast<float4*>(kc_smem);
+    float* pw = reinterpret_cast<float*>(kc_smem);
+    float2* s_w = reinterpret_cast<float2*>(kc_smem) + kL * 16;
+    const int tid = threadIdx.x, lane16 = tid & 15, item = tid >> 4;
+    const int ch8 = lane16 >> 1, pol = lane16 & 1;
+    for (int i = tid; i < 512; i += 256) s_w[i] = p.tab_w[i];
+    __syncthreads();
+
+    const int nstrips = N / 8;
+    const int nprod = nprod_of_mode(p.mode);
+    const bool own_only = p.mode == B2F_POL_P0 || p.mode == B2F_POL_P1 || p.mode == B2F_POL_I || p.mode == B2F_POL_PPQQ;
+    const int64_t nwork = (p.gb_end - p.gb_begin) * nstrips;
+    for (int64_t w = blockIdx.x; w < nwork; w += gridDim.x) {
+        const int64_t lb = w / nstrips;
+        const int64_t gb = p.gb_begin + lb;
+        const int ifi = (int)(gb / p.nblk);
+        const int64_t blk = gb % p.nblk;
+        const int strip = (int)(w % nstrips);
+        const int c = strip * 8 + ch8;
+        const float2* Z = p.spec + lb * (int64_t)kL * R;
+        float2 xA[16], xB[16];                       // un-mixed bins k2 = 32 a + item (+ 16)
+#pragma unroll
+        for (int a = 0; a < 16; ++a) {
+            xA[a] = kc_load_unmixed<R>(Z, 32 * a + item, c, pol);
+            xB[a] = kc_load_unmixed<R>(Z, 32 * a + item + 16, c, pol);
+        }
+        for (int t = 0; t < p.ndm; ++t) {
+            const int slot = t * p.nif + ifi;
+            const float2* H = p.chirp + (int64_t)slot * kL * N;
+            float2 vA[16], vB[16];
+#pragma unroll
+            for (int a = 0; a < 16; ++a) {
+                vA[a] = cmul(xA[a], H[(int64_t)(32 * a + item) * N + c]);
+                vB[a] = cmul(xB[a], H[(int64_t)(32 * a + item + 16) * N + c]);
+            }
+            kc_backward_detect<R>(vA, vB, p, data4, pw, s_w, nprod, own_only, slot, blk, strip);
+        }
     }
 }
 
@@ -2205,7 +2358,7 @@ static __global__ void ks_final(const double2* __restrict__ partial, int nsplit,
 
 // ================================================================== kernel 5b: requantise + flip + splice
 // One thread = 4 consecutive output channels of one output row.  The band flip of USB
-// subbands and the splice order are index arithmetic on the load side.
+// subbands, the splice order and the trial-major layout of a row with trial DMs are index arithmetic on the load side.
 struct KQParams {
     const float* F; int64_t F_if_stride;
     const float* mean; const float* scale;        // [nif][nprod*nchan]
@@ -2216,6 +2369,8 @@ struct KQParams {
     int if_order[B2F_MAX_IF];
     int flip[B2F_MAX_IF];                          // 1: channel reversal (USB)
     float inv_digi_sigma;                          // 1 / (sigmas spanned by half the output range): 1/6 for digifil
+    int trial_row_elems;                           // elements of one trial's slice of a row (= out_row_elems without trials);
+                                                   // trial k reads F / mean / scale slots k * nif + IF
 };
 
 __device__ __forceinline__ float quant(float y, float dscale, float dmean, float dmax) {
@@ -2228,7 +2383,9 @@ static __global__ void kq_quantise(const KQParams p) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= p.rows * quads_per_row) return;
     const int64_t row = i / quads_per_row;
-    const int j = (int)(i % quads_per_row) * 4;
+    const int jr = (int)(i % quads_per_row) * 4;   // element of the whole row
+    const int trial = jr / p.trial_row_elems;
+    const int j = jr - trial * p.trial_row_elems;  // element of this trial's slice
     int tile, prod, k;
     if (p.pol_major) {
         prod = j / (p.nif * p.nchan);
@@ -2240,10 +2397,11 @@ static __global__ void kq_quantise(const KQParams p) {
         k = j % p.nchan;
     }
     const int ifi = p.if_order[tile];
+    const int slot = trial * p.nif + ifi;
     const int ncol = p.nprod * p.nchan;
-    const float* f = p.F + ifi * p.F_if_stride + row * (int64_t)ncol + prod * p.nchan;
-    const float* mu = p.mean + ifi * ncol + prod * p.nchan;
-    const float* sc = p.scale + ifi * ncol + prod * p.nchan;
+    const float* f = p.F + slot * p.F_if_stride + row * (int64_t)ncol + prod * p.nchan;
+    const float* mu = p.mean + slot * ncol + prod * p.nchan;
+    const float* sc = p.scale + slot * ncol + prod * p.nchan;
     float y[4];
 #pragma unroll
     for (int a = 0; a < 4; ++a) {
@@ -2257,21 +2415,21 @@ static __global__ void kq_quantise(const KQParams p) {
         uint32_t w = 0;
 #pragma unroll
         for (int a = 0; a < 4; ++a) w |= (uint32_t)quant(y[a], 127.5f * p.inv_digi_sigma, 127.5f, 255.f) << (8 * a);
-        *reinterpret_cast<uint32_t*>(orow + j) = w;
+        *reinterpret_cast<uint32_t*>(orow + jr) = w;
     } else if (p.out_nbit == 16) {
         ushort4 w;
         w.x = (unsigned short)quant(y[0], 32768.0f * p.inv_digi_sigma, 32768.0f, 65535.f);
         w.y = (unsigned short)quant(y[1], 32768.0f * p.inv_digi_sigma, 32768.0f, 65535.f);
         w.z = (unsigned short)quant(y[2], 32768.0f * p.inv_digi_sigma, 32768.0f, 65535.f);
         w.w = (unsigned short)quant(y[3], 32768.0f * p.inv_digi_sigma, 32768.0f, 65535.f);
-        *reinterpret_cast<ushort4*>(orow + 2 * (int64_t)j) = w;
+        *reinterpret_cast<ushort4*>(orow + 2 * (int64_t)jr) = w;
     } else if (p.out_nbit == 2) {
         uint32_t w = 0;
 #pragma unroll
         for (int a = 0; a < 4; ++a) w |= (uint32_t)quant(y[a], 1.0f, 1.5f, 3.f) << (2 * a);
-        orow[j / 4] = (uint8_t)w;
+        orow[jr / 4] = (uint8_t)w;
     } else {
-        *reinterpret_cast<float4*>(orow + 4 * (int64_t)j) = make_float4(y[0], y[1], y[2], y[3]);
+        *reinterpret_cast<float4*>(orow + 4 * (int64_t)jr) = make_float4(y[0], y[1], y[2], y[3]);
     }
 }
 #endif

@@ -10,7 +10,7 @@ cudaError_t b2f_launch_kb(int R, int mode, const b2f::KBParams& p, int grid, cud
 cudaError_t b2f_launch_kr(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);     // [pair][row][2] blocks, R != 256
 cudaError_t b2f_launch_kr_part0(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);
 cudaError_t b2f_launch_kr_part1(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);
-cudaError_t b2f_launch_kc(int R, const b2f::KCParams& p, int grid, cudaStream_t st);
+cudaError_t b2f_launch_kc(int R, const b2f::KCParams& p, bool trials, int grid, cudaStream_t st);   // trials: kc_dedisp_trials
 cudaError_t b2f_launch_ka_2(int R, bool fwd_only, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
 cudaError_t b2f_launch_ka_8(int R, bool fwd_only, const b2f::KAParams& p, unsigned grid, cudaStream_t st);
 cudaError_t b2f_launch_kb_part0(int R, int mode, const b2f::KBParams& p, int grid, cudaStream_t st);   // R = 16, 32, 64

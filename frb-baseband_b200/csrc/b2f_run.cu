@@ -253,7 +253,6 @@ extern "C" int b2f_run_scan(b2f_plan* pl, int nfiles, const char* const* vdif_pa
     }
     const bool stats_only = io.stats_only != 0;
     const bool in_parts = io.part_count > 1;
-    if (!out_path && !stats_only) return failf(B2F_EINVAL, "null output path");
     if (in_parts && (io.part_index < 0 || io.part_index >= io.part_count)) return failf(B2F_EINVAL, "part_index out of range");
     if (in_parts && stats_only) return failf(B2F_EINVAL, "stats_only measures the head of the whole window: do not combine it with parts");
     b2f_params prm;
@@ -262,6 +261,22 @@ extern "C" int b2f_run_scan(b2f_plan* pl, int nfiles, const char* const* vdif_pa
     if (rc) return rc;
     rc = b2f_get_geometry(pl, &g);
     if (rc) return rc;
+    // trial DMs: one file per trial, each with that trial's slice of every row
+    const bool trials = prm.ndm > 0;
+    if (trials) {
+        if (out_path) return failf(B2F_EINVAL, "a plan with trial DMs writes trial_out_paths: out_path must be NULL");
+        if (in_parts) return failf(B2F_EUNSUPPORTED, "a scan with trial DMs cannot be processed in parts");
+        if (!stats_only) {
+            if (!io.trial_out_paths) return failf(B2F_EINVAL, "a plan with trial DMs needs trial_out_paths (one file per trial)");
+            for (int k = 0; k < prm.ndm; ++k)
+                if (!io.trial_out_paths[k]) return failf(B2F_EINVAL, "null trial output path");
+        }
+    } else {
+        if (io.trial_out_paths) return failf(B2F_EINVAL, "trial_out_paths needs a plan with trial DMs");
+        if (!out_path && !stats_only) return failf(B2F_EINVAL, "null output path");
+    }
+    const int nout = trials ? prm.ndm : 1;
+    auto path_of = [&](int k) { return trials ? io.trial_out_paths[k] : out_path; };
     // Placement by header time works inside one push: a frame whose header time lies beyond the push is dropped and
     // never presented again, while this runner reads files positionally chunk by chunk -- after a gap every later
     // chunk would lose its last frames.  Whole files are digifil's positional reader (process_vdif.py:157-161).
@@ -346,29 +361,35 @@ extern "C" int b2f_run_scan(b2f_plan* pl, int nfiles, const char* const* vdif_pa
     }
 
     // ---- output: an existing FIFO (base2fil.sh:348-349) is opened as it is, never unlinked (process_vdif.py:146-149)
-    int ofd = -1;
+    std::vector<int> ofds;                    // one file, or one per trial DM
     bool out_is_fifo = false;
     bool positioned = false;                  // parts write at their final offset (pwrite) into a file nobody truncates
-    if (!stats_only) {
+    for (int k = 0; k < nout && !stats_only; ++k) {
+        const char* op = path_of(k);
         struct stat st;
-        const bool fifo = stat(out_path, &st) == 0 && S_ISFIFO(st.st_mode);
+        const bool fifo = stat(op, &st) == 0 && S_ISFIFO(st.st_mode);
         if (fifo && in_parts) return failf(B2F_EINVAL, "parts of a scan cannot be written to a FIFO");
+        // the trial files are written in lockstep: a reader that drains one pipe after another would deadlock the scan
+        if (fifo && trials) return failf(B2F_EINVAL, std::string(op) + ": trial DM outputs must be regular files, not FIFOs");
         out_is_fifo = fifo;
+        int ofd = -1;
         if (fifo) {
-            ofd = open(out_path, O_WRONLY);
+            ofd = open(op, O_WRONLY);
 #ifdef F_SETPIPE_SZ
             // what setfifo.perl does for every FIFO of the splice list (setfifo.perl:10, base2fil.sh:417-419): 1 MiB pipe
             if (ofd >= 0) (void)fcntl(ofd, F_SETPIPE_SZ, 1048576);
 #endif
         } else {
-            ofd = open(out_path, in_parts ? (O_WRONLY | O_CREAT) : (O_WRONLY | O_CREAT | O_TRUNC), 0644);
+            ofd = open(op, in_parts ? (O_WRONLY | O_CREAT) : (O_WRONLY | O_CREAT | O_TRUNC), 0644);
         }
-        if (ofd < 0) return failf(B2F_EINVAL, std::string("cannot open ") + out_path + " for writing: " + strerror(errno));
+        if (ofd < 0) return failf(B2F_EINVAL, std::string("cannot open ") + op + " for writing: " + strerror(errno));
         own.fds.push_back(ofd);
+        ofds.push_back(ofd);
         positioned = in_parts;
     }
+    const int ofd = ofds.empty() ? -1 : ofds[0];
     int64_t bytes_out = 0;
-    off_t out_pos = 0;
+    off_t out_pos = 0, hdr_bytes = 0;
     if (!stats_only) {
         double top = prm.freq_mhz[0];
         for (int i = 1; i < prm.nif; ++i) top = std::max(top, prm.freq_mhz[i]);
@@ -392,15 +413,22 @@ extern "C" int b2f_run_scan(b2f_plan* pl, int nfiles, const char* const* vdif_pa
         fh.nifs = g.nprod;
         fh.refdm = io.refdm;
         fh.write_refdm = io.write_refdm;
-        uint8_t hb[1024];
-        size_t hn = 0;
-        rc = b2f_sigproc_header(&fh, hb, sizeof hb, &hn);
-        if (rc) return rc;
-        if (!positioned || io.part_index == 0) {
-            if (!write_fully(ofd, hb, hn, positioned ? 0 : -1)) return failf(B2F_EINVAL, std::string("write failed: ") + strerror(errno));
-            bytes_out += (int64_t)hn;
+        for (int k = 0; k < nout; ++k) {
+            if (trials) {
+                fh.refdm = prm.dm_trials[k];
+                fh.write_refdm = 1;
+            }
+            uint8_t hb[1024];
+            size_t hn = 0;
+            rc = b2f_sigproc_header(&fh, hb, sizeof hb, &hn);
+            if (rc) return rc;
+            if (!positioned || io.part_index == 0) {
+                if (!write_fully(ofds[k], hb, hn, positioned ? 0 : -1)) return failf(B2F_EINVAL, std::string("write failed: ") + strerror(errno));
+                bytes_out += (int64_t)hn;
+            }
+            hdr_bytes = (off_t)hn;                                   // the same length for every trial: refdm is always written
+            out_pos = (off_t)hn + (off_t)(row0 * g.row_bytes);
         }
-        out_pos = (off_t)hn + (off_t)(row0 * g.row_bytes);
     }
 
     // ---- pinned ring + output buffers
@@ -473,6 +501,8 @@ extern "C" int b2f_run_scan(b2f_plan* pl, int nfiles, const char* const* vdif_pa
         for (auto& t : readers) if (t.joinable()) t.join();
     };
 
+    std::vector<uint8_t> gather(trials && !stats_only ? (size_t)max_rows * (size_t)g.trial_row_bytes : 0);   // the writer's, per trial
+
     // ---- feed the plan; rows of chunk k are written while chunk k+1 is on the GPU
     int64_t rows_total = 0, frames_done = 0;
     double t_wait_read = 0, t_wait_gpu = 0, t_write = 0;
@@ -497,7 +527,16 @@ extern "C" int b2f_run_scan(b2f_plan* pl, int nfiles, const char* const* vdif_pa
             // (or tmpfs) allocates and fills pages at about 3 GB/s, which at 100x real time is what the whole runner waits
             // for (320 MB of rows per 20 s of C2).  A FIFO is a byte stream: one writer, in order.
             bool ok = true;
-            if (!W.failed) {
+            if (!W.failed && trials) {
+                // each trial's slice of every row, gathered into one contiguous piece per file
+                const int64_t trb = g.trial_row_bytes, nr = (int64_t)(job.second / (size_t)g.row_bytes);
+                const off_t tpos = hdr_bytes + (off_t)((out_pos - hdr_bytes) / g.row_bytes * trb);   // rows written so far
+                for (int k = 0; k < nout && ok; ++k) {
+                    const uint8_t* src = outb[job.first] + k * trb;
+                    for (int64_t r = 0; r < nr; ++r) memcpy(gather.data() + r * trb, src + r * g.row_bytes, (size_t)trb);
+                    ok = write_fully(ofds[k], gather.data(), (size_t)(nr * trb), tpos);
+                }
+            } else if (!W.failed) {
                 const uint8_t* src = outb[job.first];
                 const size_t n = job.second;
                 constexpr int kPar = 4;

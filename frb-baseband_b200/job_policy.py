@@ -8,15 +8,19 @@ samples up to the wanted time resolution.
 
 `gpu_plan` is the B200 addition: with in-channel coherent dedispersion (b2f_params.coherent) the
 smearing term vanishes, so the channel count is set by what the search downstream wants rather than
-by the DM.
+by the DM.  `coherent_search_plan` is its search form for an unknown DM: a ladder of trial DMs, each
+coherently dedispersed (b2f_params.ndm / dm_trials), spaced so that the smearing left inside a channel
+never exceeds the time resolution.
 """
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass
 
 K_SMEAR_US = 8.3            # submit_job.py:60 (us per MHz per pc/cc at 1 GHz)
 MAX_BAND_CHANNELS = 2 ** 13   # submit_job.py:63
 UNKNOWN_DM = 1500.0         # submit_job.py:52-54: Heimdall's search ceiling when the source has no DM
+MAX_TRIAL_DMS = 64          # B2F_MAX_DM of include/b2f.h
 FLAG_DIR = "/data1/franz/fetch/Standard/"   # submit_job.py:38
 
 
@@ -30,6 +34,7 @@ class ChannelPlan:
     f_max_mhz: int
     coherent: bool = False
     dm: float = 0.0
+    dm_trials: tuple = ()       # coherent trial DMs (coherent_search_plan), ascending
 
     def flag_file(self, telescope: str, flag_dir: str = FLAG_DIR) -> str:
         """RFI flag file FETCH is pointed at: submit_job.py:117"""
@@ -110,6 +115,29 @@ def gpu_plan(dm: float | None, fref_mhz: float, if_mhz: float, nif: int, *, log2
     f_min_ghz = (fref_mhz - if_mhz) / 1000
     band = float(nif) * if_mhz
     return _finish(nchan_if * nif, nchan_if, 2 ** log2_t_res_us, f_min_ghz, if_mhz, band, coherent=True, dm=dm)
+
+
+def coherent_search_plan(dm_max: float | None, fref_mhz: float, if_mhz: float, nif: int, *, log2_t_res_us: int = 6,
+                         nchan_if: int = 128) -> ChannelPlan:
+    """Search for an unknown DM with coherent dedispersion at a ladder of trial DMs, all in one pass over the baseband.
+
+    A channel dedispersed at DM d keeps 8.3 us * |DM - d| * chbw / f_min^3 of smearing at the bottom of the band.  Trials
+    `step` apart with step = 2 t_res f_min^3 / (8.3 chbw), at step/2 + k step, leave at most t_res for every DM in
+    [0, dm_max].  More than MAX_TRIAL_DMS trials is a ValueError: use fewer channels' worth of time resolution or a lower
+    dm_max."""
+    dm_max = UNKNOWN_DM if dm_max is None else float(dm_max)
+    if not dm_max > 0:
+        raise ValueError(f"dm_max = {dm_max}: must be > 0")
+    f_min_ghz = (fref_mhz - if_mhz) / 1000
+    band = float(nif) * if_mhz
+    t_res = 2 ** log2_t_res_us
+    chbw = if_mhz / nchan_if
+    step = 2 * t_res * f_min_ghz ** 3 / (K_SMEAR_US * chbw)
+    n = max(1, math.ceil(dm_max / step - 1e-9))
+    if n > MAX_TRIAL_DMS:
+        raise ValueError(f"{n} trial DMs {step:.1f} apart are needed up to DM {dm_max} at {t_res} us, at most {MAX_TRIAL_DMS} fit one plan")
+    trials = tuple(step / 2 + k * step for k in range(n))
+    return _finish(nchan_if * nif, nchan_if, t_res, f_min_ghz, if_mhz, band, coherent=True, dm=dm_max, dm_trials=trials)
 
 
 def create_config_argv(plan: ChannelPlan, *, vex: str, source: str, telescope: str, scan: str, config_file: str,

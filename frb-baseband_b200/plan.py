@@ -51,6 +51,7 @@ class PlanConfig:
     stream: int | None = None
     dm: float = 0.0                          # digifil -D
     coherent: bool = False                   # digifil -F nchan:D
+    dm_trials: list[float] | None = None     # coherent dedispersion at each of these DMs in one pass (dm stays 0)
     raw_word_bits: int = 0                   # 16/32/64: one raw multi-BBC VDIF stream, corner turn on the GPU
     raw_bits: list | None = None             # per IF: 4 source bit positions (spif2file recipe)
     raw_format: int = 0                      # 0 VDIF frames, 1 Mark5B disk frames (16 B header, 10000 B payload)
@@ -96,6 +97,12 @@ class Plan:
             p.if_order[i] = order[i]
         p.dm = cfg.dm
         p.coherent = int(cfg.coherent)
+        trials = list(cfg.dm_trials or [])
+        if len(trials) > _lib.B2F_MAX_DM:
+            raise B2FError(_lib.EINVAL, f"at most {_lib.B2F_MAX_DM} trial DMs")
+        p.ndm = len(trials)
+        for k, d in enumerate(trials):
+            p.dm_trials[k] = float(d)
         p.profile = int(cfg.profile)
         p.raw_word_bits = cfg.raw_word_bits
         p.raw_format = cfg.raw_format
@@ -122,6 +129,9 @@ class Plan:
         self.geometry = g
         self.nprod = g.nprod
         self.row_bytes = g.row_bytes
+        #: trial DMs of the plan (1 without trials); a row holds ndm slices of trial_row_bytes, trial-major
+        self.ndm = g.ndm
+        self.trial_row_bytes = g.trial_row_bytes
         self.chunk_frames = g.chunk_frames
         self.chunk_rows = g.chunk_rows
         self.tsamp_s = g.tsamp_s
@@ -207,7 +217,7 @@ class Plan:
     def wait(self, ticket: int):
         _lib.check(_lib.lib().b2f_wait(self._h, int(ticket)))
 
-    def run_scan(self, paths, out_path: str, *, start_s: float = 0.0, nsec: float | None = None,
+    def run_scan(self, paths, out_path, *, start_s: float = 0.0, nsec: float | None = None,
                  source_name: str = "unknown", rawdatafile: str | None = None, telescope_id: int = 0,
                  machine_id: int = 0, src_raj: float = 0.0, src_dej: float = 0.0, refdm: float | None = None,
                  ring: int = 0, readers_per_file: int = 0, part: tuple[int, int] | None = None,
@@ -215,7 +225,8 @@ class Plan:
         """Files in, filterbank file out, entirely inside libb2f (b2f_run_scan): threaded readers, pinned ring,
         pipelined pushes/pulls.  `paths`: one split VDIF file per IF in plan order (or the one raw recording).
         `part=(k, n)`: only time segment k of n, written at its final offset of `out_path` (needs set_rescale
-        unless keep_bandpass); `stats_only`: measure the first rescale interval, write nothing."""
+        unless keep_bandpass); `stats_only`: measure the first rescale interval, write nothing.  A plan with trial DMs
+        takes a list of `ndm` output paths, one filterbank per trial with refdm = its DM."""
         io = _lib.ScanIO()
         io.struct_size = C.sizeof(_lib.ScanIO)
         io.start_s = float(start_s)
@@ -230,6 +241,12 @@ class Plan:
         io.readers_per_file = readers_per_file
         io.part_index, io.part_count = part if part else (0, 0)
         io.stats_only = int(stats_only)
+        if isinstance(out_path, (list, tuple)):
+            if len(out_path) != self.ndm or not self.cfg.dm_trials:
+                raise B2FError(_lib.EINVAL, f"a list of output paths needs a plan with {len(out_path)} trial DMs")
+            tarr = (C.c_char_p * len(out_path))(*[os.fsencode(p) for p in out_path])
+            io.trial_out_paths = C.cast(tarr, C.POINTER(C.c_char_p))
+            out_path = None
         arr = (C.c_char_p * len(paths))(*[os.fsencode(p) for p in paths])
         res = _lib.ScanResult()
         _lib.check(_lib.lib().b2f_run_scan(self._h, len(paths), arr, None if out_path is None else os.fsencode(out_path),
@@ -249,11 +266,14 @@ class Plan:
         return c.as_dict()
 
     def rescale(self):
-        n = self.nif * self.nprod * self.cfg.nchan
+        """mean, scale as [nif, nprod, nchan]; [ndm, nif, nprod, nchan] for a plan with trial DMs."""
+        n = self.ndm * self.nif * self.nprod * self.cfg.nchan
         mean = np.empty(n, np.float32)
         scale = np.empty(n, np.float32)
         _lib.check(_lib.lib().b2f_get_rescale(self._h, mean.ctypes.data, scale.ctypes.data))
         shp = (self.nif, self.nprod, self.cfg.nchan)
+        if self.cfg.dm_trials:
+            shp = (self.ndm,) + shp
         return mean.reshape(shp), scale.reshape(shp)
 
     def set_rescale(self, mean: np.ndarray | None, scale: np.ndarray | None = None):
@@ -263,7 +283,7 @@ class Plan:
             return
         m = np.ascontiguousarray(mean, np.float32).reshape(-1)
         s = np.ascontiguousarray(scale, np.float32).reshape(-1)
-        assert m.size == s.size == self.nif * self.nprod * self.cfg.nchan
+        assert m.size == s.size == self.ndm * self.nif * self.nprod * self.cfg.nchan
         _lib.check(_lib.lib().b2f_set_rescale(self._h, m.ctypes.data, s.ctypes.data))
 
     def kernel_times(self) -> dict:
@@ -285,6 +305,12 @@ class Plan:
         buf = np.empty(nbytes, np.uint8)
         _lib.check(_lib.lib().b2f_debug_copy(self._h, which, buf.ctypes.data, nbytes, None))
         return buf.view(dtype)
+
+    def trial_rows(self, raw: np.ndarray) -> np.ndarray:
+        """[rows, row_bytes] uint8 -> [ndm, rows, trial_row_bytes] view: trial k's rows as a single-DM plan writes them."""
+        raw = np.ascontiguousarray(raw, np.uint8).reshape(-1, self.row_bytes)
+        v = raw.reshape(raw.shape[0], self.ndm, self.trial_row_bytes)
+        return v.transpose(1, 0, 2)
 
     def view_rows(self, raw: np.ndarray) -> np.ndarray:
         """[rows, row_bytes] uint8 -> [rows, elems] in the output sample type."""

@@ -48,6 +48,10 @@ _CLI = [
     (("--coherent_dm",), dict(type=float, default=0.0,
                               help="extension: coherently dedisperse inside each channel at this DM "
                                    "(run_digifil's dm/coherent arguments, which the reference CLI never sets)"), _D),
+    (("--coherent_numdms",), dict(type=int, default=1,
+                                  help="extension: with N >= 2, coherent dedispersion at the N trial DMs coherent_dm + k "
+                                       "coherent_dmstep in one pass, one <stem>_DM<dm>.fil per trial (%(default)s)"), _D),
+    (("--coherent_dmstep",), dict(type=float, default=0.0, help="extension: DM step of the coherent trials"), _D),
     (("--do_prepdata",), dict(action="store_true", help="run PRESTO prepdata/prepsubband afterwards"), _P),
     (("--ncpus",), dict(type=int, default=1, help="1: prepdata, >1: prepsubband"), _P),
     (("--dm",), dict(type=float, default=None, help="DM for prepdata (default: psrcat)"), _P),
@@ -136,10 +140,46 @@ def _output_path(hdr, fil_out_dir, overwrite):
     return fil
 
 
+def coherent_trials(dm, numdms, dmstep):
+    """Trial DMs of --coherent_dm/--coherent_numdms/--coherent_dmstep (prepsubband's -lodm/-numdms/-dmstep), or None
+    for a single DM (numdms 1)."""
+    if numdms < 1:
+        raise InputError(f"--coherent_numdms {numdms}: must be >= 1")
+    if numdms == 1:
+        return None
+    if not dmstep > 0:
+        raise InputError("--coherent_numdms >= 2 needs --coherent_dmstep > 0")
+    if dm < 0:
+        raise InputError("--coherent_dm must be >= 0")
+    return [dm + k * dmstep for k in range(numdms)]
+
+
+def trial_output_paths(hdr, fil_out_dir, dm_trials):
+    """<stem>_DM<dm:.2f>.fil per trial DM, in fil_out_dir (or beside the .hdr)."""
+    fil = hdr[:-4] + ".fil" if hdr.endswith(".hdr") else hdr.replace(".hdr", ".fil")
+    if fil_out_dir is not None:
+        fil = "{0}/{1}".format(fil_out_dir, os.path.basename(fil))
+    stem = fil[:-4]
+    return ["{0}_DM{1:.2f}.fil".format(stem, d) for d in dm_trials]
+
+
 def run_digifil(hdr, fil_out_dir=None, start=1, nsecs=120, nchan=128, overwrite=False, pol=2, nbit=8,
-                tscrunch=1, nthreads=1, dm=0.0, coherent=False, keepBP=False, device=0):
-    """Baseband -> filterbank for the subband described by `hdr`; returns the .fil path."""
-    fil = _output_path(hdr, fil_out_dir, overwrite)
+                tscrunch=1, nthreads=1, dm=0.0, coherent=False, keepBP=False, device=0, dm_trials=None):
+    """Baseband -> filterbank for the subband described by `hdr`; returns the .fil path.  With `dm_trials` (a list of
+    DMs) one pass writes a coherently dedispersed filterbank per trial and the list of their paths is returned."""
+    if dm_trials is not None:
+        fils = trial_output_paths(hdr, fil_out_dir, dm_trials)
+        for f in fils:
+            if os.path.exists(f):
+                if not overwrite:
+                    raise InputError("Filterbankfile {0} exists already. Delete first or set --force to overwrite".format(f))
+                if stat.S_ISFIFO(os.stat(f).st_mode):
+                    raise InputError("{0}: trial DM outputs must be regular files, not FIFOs".format(f))
+                os.remove(f)
+        fil = fils
+        dm, coherent = 0.0, True
+    else:
+        fil = _output_path(hdr, fil_out_dir, overwrite)
     if nbit not in (2, 8, 16, -32):
         raise InputError(f"nbit={nbit} not in supported values of [2, 8, 16, -32]. ")
     if pol not in (0, 1, 2, 3, 4):
@@ -150,8 +190,11 @@ def run_digifil(hdr, fil_out_dir=None, start=1, nsecs=120, nchan=128, overwrite=
 
     kv = read_hdr(hdr)
     datafile, freq, bw = kv["DATAFILE"], float(kv["FREQ"]), float(kv["BW"])
+    dedisp = "D -D {0}".format(dm) if (coherent and dm > 0) else reference_freq_res(nchan)
+    if dm_trials is not None:
+        dedisp = "D -D {0}".format(",".join("{0:.2f}".format(d) for d in dm_trials))
     print("running b2f -b{0} -S{1} -T{2} -t {3} -o {4} {5} pol={6} -F{7}:{8}{9} (libb2f.so, cuda:{10})".format(
-        nbit, start, nsecs, tscrunch, fil, hdr, pol, nchan, "D -D {0}".format(dm) if (coherent and dm > 0) else reference_freq_res(nchan),
+        nbit, start, nsecs, tscrunch, " ".join(fil) if dm_trials is not None else fil, hdr, pol, nchan, dedisp,
         " -I0" if keepBP else "", device))
     try:
         with open(datafile, "rb") as src:
@@ -162,7 +205,8 @@ def run_digifil(hdr, fil_out_dir=None, start=1, nsecs=120, nchan=128, overwrite=
         cfg = PlanConfig(nchan=nchan, bw_mhz=[bw], freq_mhz=[freq], tscrunch=max(1, tscrunch),
                          pol_mode=pol_mode_from_reference(pol), out_nbit=nbit, in_nbit=info.nbit,
                          frame_bytes=info.frame_bytes, header_bytes=info.header_bytes, keep_bandpass=keepBP,
-                         device=device, dm=float(dm), coherent=bool(coherent and dm > 0.0),
+                         device=device, dm=float(dm), coherent=bool(coherent and (dm > 0.0 or dm_trials is not None)),
+                         dm_trials=None if dm_trials is None else [float(d) for d in dm_trials],
                          # the reference passes -2 (:157,160): DSPSR's dynamic 2-bit levels; this build defaults to the
                          # static optimal levels, B2F_DECODE_MODE=ja98 selects the reference-faithful unpacker
                          decode_mode=_lib.DECODE_JA98 if os.environ.get("B2F_DECODE_MODE", "").lower() == "ja98" else _lib.DECODE_STATIC)
@@ -172,7 +216,8 @@ def run_digifil(hdr, fil_out_dir=None, start=1, nsecs=120, nchan=128, overwrite=
             c = pl.run_scan([datafile], fil, start_s=start, nsec=nsecs, source_name=kv.get("SOURCE", "unknown"),
                             telescope_id=sigproc.TELESCOPE_IDS.get(kv.get("TELESCOPE", "").lower(), 0),
                             src_raj=sigproc.sexagesimal_to_sigproc(kv.get("RA")),
-                            src_dej=sigproc.sexagesimal_to_sigproc(kv.get("DEC")), refdm=dm)["counters"]
+                            src_dej=sigproc.sexagesimal_to_sigproc(kv.get("DEC")),
+                            refdm=None if dm_trials is not None else dm)["counters"]
         if c["frames_invalid"] or c["frames_with_fill"] or c["frames_badhdr"]:
             print("b2f: masked {frames_invalid} invalid, {frames_with_fill} fill-pattern and {frames_badhdr} "
                   "malformed frames".format(**c), file=sys.stderr)
@@ -217,9 +262,12 @@ def main(argv=None):
     if a.hdr_only:
         print("Not creating filterbanks. Hdr files done.")
         return 0
+    trials = coherent_trials(a.coherent_dm, a.coherent_numdms, a.coherent_dmstep)
+    if a.do_prepdata and trials is not None:
+        raise InputError("--do_prepdata takes one filterbank: not with --coherent_numdms >= 2")
     fil = run_digifil(hdr, a.fil_out_dir, a.start, a.nsec, a.nchan, overwrite=a.force, pol=a.pol, nbit=a.nbit,
                       tscrunch=a.tscrunch, nthreads=a.nthreads, keepBP=a.keepBP, device=a.device,
-                      dm=a.coherent_dm, coherent=a.coherent_dm > 0.0)
+                      dm=a.coherent_dm, coherent=a.coherent_dm > 0.0, dm_trials=trials)
     if a.do_prepdata:
         prepdata(fil, a.dm if a.dm is not None else psr_info(a.psrname)[2], zerodm=a.nozerodm, clip=a.clip,
                  dm2=a.dm2, dmstep=a.dmstep, ncpus=a.ncpus)

@@ -31,6 +31,7 @@ extern "C" {
 
 #define B2F_VERSION 100            /* 0.1.0 */
 #define B2F_MAX_IF 32
+#define B2F_MAX_DM 64              /* trial DMs of one coherent search plan */
 
 struct b2f_plan;                   /* opaque: created by b2f_plan_create, owned by the library */
 
@@ -131,6 +132,12 @@ typedef struct b2f_params {
     double digi_sigma;             /* D9: half the output range spans this many sigma (digifil: 6); 0 = 6       */
     int32_t raw_format;            /* enum b2f_raw_format; only read when raw_word_bits != 0                    */
     int32_t reserved0;             /* must be 0                                                                 */
+    /* ---- coherent dedispersion at several trial DMs in one pass: the spectrum of every overlap-save block is computed once
+       and each trial applies its own chirp to it, so one plan writes ndm filterbanks.  Needs coherent = 1 and dm = 0;
+       trials finite, >= 0, strictly increasing, the largest > 0.  freq_res, nfilt and the push size follow the largest
+       trial by the single-DM rule, and its refusals apply (smearing beyond 4096 points, nchan 4096). */
+    int32_t ndm;                   /* 0: one DM, taken from dm; 1..B2F_MAX_DM: trial DMs dm_trials[0..ndm-1]          */
+    double dm_trials[B2F_MAX_DM];
 } b2f_params;
 
 typedef struct b2f_geometry {
@@ -140,12 +147,15 @@ typedef struct b2f_geometry {
     int64_t chunk_rows;            /* output time samples produced per full push              */
     int64_t block_samples;         /* M = 2*nchan*freq_res time samples                       */
     int64_t samples_per_frame;
-    int64_t row_bytes;             /* bytes of one output time sample (all IFs, all products) */
+    int64_t row_bytes;             /* bytes of one output time sample (all trials, IFs, products) = ndm * trial_row_bytes */
     int32_t nprod;                 /* detected streams (SIGPROC nifs)                         */
     int32_t freq_res;
     double tsamp_s;
     int64_t interval_rows;         /* rows held before the first rescale is frozen            */
     int32_t nfilt_pos, nfilt_neg;  /* overlap-save samples discarded per block and channel (dedispersion) */
+    int32_t ndm;                   /* trial DMs; 1 when trials are off                        */
+    int64_t trial_row_bytes;       /* bytes of one trial's slice of a row: trial k starts at k * trial_row_bytes and holds
+                                      exactly the row a single-DM plan at dm_trials[k] writes (either splice layout)      */
 } b2f_geometry;
 
 typedef struct b2f_counters {
@@ -199,11 +209,13 @@ int b2f_pull(struct b2f_plan* plan, void* out, int64_t max_rows, int out_on_devi
  * owns part of the band drops its tile into the wider spliced rows of the rank that owns the file --
  * `out` may be that rank's memory mapped over NVLink (the in-GPU form of base2fil.sh:422's splice). */
 int b2f_pull_strided(struct b2f_plan* plan, void* out, int64_t max_rows, int64_t row_pitch_bytes, int64_t* nrows);
+/* (B2F_EUNSUPPORTED for a plan with trial DMs) */
 
 int b2f_sync(struct b2f_plan* plan);
 int b2f_reset(struct b2f_plan* plan);        /* new scan, same parameters */
 int b2f_get_counters(struct b2f_plan* plan, b2f_counters* out);
-/* mean/scale the digitiser applies: arrays of nif*nprod*nchan floats, natural channel order */
+/* mean/scale the digitiser applies: arrays of ndm*nif*nprod*nchan floats (ndm = 1 without trials), trial-major,
+ * natural channel order */
 int b2f_get_rescale(struct b2f_plan* plan, float* mean, float* scale);
 /* Freeze the digitiser's mean/scale from outside instead of measuring them on the first rescale interval: a scan
  * cut into time segments (several GPUs, or several calls) must requantise every segment with the statistics of the
@@ -274,6 +286,10 @@ typedef struct b2f_scan_io {
                                       the plan needs b2f_set_rescale first (statistics of the scan's first interval) */
     int32_t stats_only;            /* 1: stop as soon as the first rescale interval is measured, write nothing
                                       (out_path may be NULL); read the result with b2f_get_rescale */
+    const char* const* trial_out_paths; /* plan with trial DMs: one regular file per trial (out_path must be NULL), each
+                                      with its own header (refdm = dm_trials[k]) and that trial's slice of every row.
+                                      FIFOs are refused (B2F_EINVAL: a reader of one of ndm pipes written in lockstep
+                                      can deadlock), and so are parts (B2F_EUNSUPPORTED) */
 } b2f_scan_io;
 
 typedef struct b2f_scan_result {
@@ -312,7 +328,7 @@ int b2f_fp32_peak(int device, double* tflops);
  * which: 0 compact payload, 1 word mask, 2 frame status, 3 block dirty flags,
  *        4 column-pass output [blk][L][R] float2 (paths 1, 2: slots of [32][R/2][16][2] float2; path 2: only the ring),
  *        5 column sums [blk][R] float2,
- *        6 eps [blk][nchan] float2, 7 detected floats of held rows [if][row][prod][chan]. */
+ *        6 eps [blk][nchan] float2, 7 detected floats of held rows [trial][if][row][prod][chan]. */
 int b2f_debug_copy(struct b2f_plan* plan, int which, void* dst, size_t nbytes, size_t* needed);
 
 #ifdef __cplusplus
