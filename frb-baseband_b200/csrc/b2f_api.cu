@@ -16,6 +16,7 @@
 #include "b2f_fused.cuh"
 #include "b2f_generic.cuh"
 #include "b2f_launch.h"
+#include "b2f_long.h"
 
 using namespace b2f;
 
@@ -88,6 +89,7 @@ struct b2f_plan {
     // coherent dedispersion (digifil -D dm -F nchan:D): overlap-save geometry and halo carry
     bool dedisp = false;
     bool generic = false;          // freq_res / nchan outside the tuned 512-point kernels
+    bool longfft = false;          // dedispersion with freq_res 8192..65536 (b2f_kl.cu)
     // tscrunch that is not a power of two, or longer than freq_res (process_vdif.py:156-158 passes any -t): the kernels
     // integrate D = the largest power of two dividing it (<= freq_res), d_Fk holds their rows and kd_sum_rows adds tsq of them
     int tsq = 1;
@@ -392,7 +394,39 @@ int push_dedisp(b2f_plan* pl, int64_t nblk, int64_t T) {
         pl->launches++;
         CU(cudaGetLastError());
     }
-    if (nblk > 0 && pl->generic) {
+    if (nblk > 0 && pl->longfft) {
+        // freq_res 8192..65536 (b2f_kl.cu): forward column transform and row FFT once, the backward part once per trial
+        const int64_t NB = pl->batch_blocks > 0 ? std::min<int64_t>(pl->batch_blocks, nbt) : nbt;
+        if ((rc = stream_levels(pl, T))) return rc;
+        KLParams kl{};
+        kl.compact = pl->d_compact; kl.compact_stride = pl->compact_stride;
+        kl.wmask = pl->d_wmask; kl.wmask_stride = pl->wmask_stride; kl.blkdirty = pl->d_blkdirty;
+        kl.levels = pl->d_levels_stream; kl.levels_stride = pl->levels_stride;
+        kl.in8_offset = pl->prm.in8_offset_mode ? 128.0f : 127.5f;
+        kl.in_nbit = pl->d_levels_stream ? 22 : (pl->bps == 2 ? 8 : 2);
+        kl.step = pl->step;
+        kl.inter = pl->d_inter; kl.spec = pl->d_spec;
+        kl.F = row_dst(pl); kl.F_if_stride = row_dst_stride(pl); kl.row0 = row_dst_row0(pl);
+        kl.R = pl->R; kl.lgR = 31 - __builtin_clz(pl->R); kl.L = pl->L; kl.lgL = 31 - __builtin_clz(pl->L);
+        kl.lgLa = 8; kl.lgLb = kl.lgL - 8; kl.M = pl->M;
+        kl.nblk = (int)nblk; kl.nif = nif; kl.D = pl->D; kl.mode = pl->prm.pol_mode;
+        kl.nfilt_pos = pl->nfilt_pos; kl.keep = pl->keep;
+        for (int64_t b0 = 0; b0 < nbt; b0 += NB) {
+            kl.gb_begin = b0; kl.gb_end = b0 + std::min(NB, nbt - b0);
+            cudaError_t le = cudaSuccess;
+            if ((rc = timed(pl, B2F_K_COLUMN, [&] { le = b2f_launch_kl_column(kl, pl->stream); }))) return rc;
+            if (le != cudaSuccess) return fail(B2F_ECUDA, std::string("long column transform: ") + cudaGetErrorString(le));
+            if ((rc = timed(pl, B2F_K_ROW, [&] { le = b2f_launch_kl_row(kl, pl->stream); }))) return rc;
+            if (le != cudaSuccess) return fail(B2F_ECUDA, std::string("long row FFT: ") + cudaGetErrorString(le));
+            for (int t = 0; t < pl->ndm; ++t) {
+                KLParams kt = kl;
+                kt.chirp = pl->d_chirp + (int64_t)t * nif * pl->L * pl->N;
+                kt.F = kl.F + (int64_t)t * nif * kl.F_if_stride;
+                if ((rc = timed(pl, B2F_K_DEDISP, [&] { le = b2f_launch_kl_back(kt, pl->stream); }))) return rc;
+                if (le != cudaSuccess) return fail(B2F_ECUDA, std::string("long dedispersion back end: ") + cudaGetErrorString(le));
+            }
+        }
+    } else if (nblk > 0 && pl->generic) {
         const int64_t NB = pl->batch_blocks > 0 ? std::min<int64_t>(pl->batch_blocks, nbt) : nbt;
         KGParams kg{};
         kg.compact = pl->d_compact; kg.compact_stride = pl->compact_stride;
@@ -825,6 +859,8 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     const int R = 2 * prm->nchan;
     if (!is_pow2(R) || R < 16 || R > 8192) return fail(B2F_EUNSUPPORTED, "nchan must be a power of two in 8..4096");
     const bool dedisp = prm->coherent && dm > 0.0;
+    // the longest transform: 4096 points, or with dedispersion as many as keep a block at 2^20 points (nchan 8..64)
+    const int long_cap = std::max(4096, (1 << 20) / R);
     // overlap-save samples discarded at each end of a block and channel: half the smearing across the lowest channel of
     // the lowest subband (8.3 us DM dnu/nu_GHz^3, the rule of submit_job.py:62) plus 10 %, rounded up to a multiple of the
     // integration factor so that every block yields whole output samples
@@ -845,11 +881,20 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
         const int nf = nfilt_half(D0);
         if (2 * nf >= L) {
             while (L < 8 * nf && L < 4096) L *= 2;
-            if (2 * nf >= L) return fail(B2F_EUNSUPPORTED, "dispersion smearing exceeds freq_res 4096 channel samples: use more channels");
+            // where 4096 points do not hold the smearing: the long-transform path, up to 2^20 points per block
+            if (2 * nf >= L) while (L < 8 * nf && L < long_cap) L *= 2;
+            if (2 * nf >= L)
+                return fail(B2F_EUNSUPPORTED, "dispersion smearing exceeds freq_res " + std::to_string(long_cap) + " channel samples at nchan " +
+                                                  std::to_string(prm->nchan) + ": use more channels");
         }
     }
-    if (!is_pow2(L) || L < 16 || L > 8192) return fail(B2F_EUNSUPPORTED, "freq_res must be a power of two in 16..8192");
-    if ((R > 4096 || L > 4096) && L != R)
+    if (!is_pow2(L) || L < 16 || L > 65536) return fail(B2F_EUNSUPPORTED, "freq_res must be a power of two in 16..8192");
+    // freq_res above 4096 (other than nchan 4096's square blocks): coherent dedispersion on the long-transform path only
+    const bool longfft = L > 4096 && L != R;
+    if (longfft && (!dedisp || L > long_cap))
+        return fail(B2F_EUNSUPPORTED, "freq_res " + std::to_string(L) + " needs coherent dedispersion and at most 2^20 points per block: freq_res <= " +
+                                          std::to_string(long_cap) + " at nchan " + std::to_string(prm->nchan));
+    if ((R > 4096 || L > 4096) && L != R && !longfft)
         return fail(B2F_EUNSUPPORTED, "nchan 4096 needs freq_res = 2 nchan (digifil -F nchan:2*nchan, process_vdif.py:162)");
     const bool generic = !(L == kL && R <= 512);        // tuned kernels: 512-point columns, rows up to 512
     const int D_user = prm->tscrunch < 1 ? 1 : prm->tscrunch;
@@ -863,7 +908,7 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     if (payload <= 0 || payload % 8) return fail(B2F_EINVAL, "frame_bytes");
     if ((dedisp || generic) && prm->in_nbit == 8 && payload % 32)
         return fail(B2F_EUNSUPPORTED, "8-bit input with coherent dedispersion, freq_res != 512 or nchan > 256 needs a payload that is a multiple of 32 bytes");
-    if (dedisp && generic && (R > 4096 || L > 4096))
+    if (dedisp && generic && !longfft && (R > 4096 || L > 4096))
         return fail(B2F_EUNSUPPORTED, "coherent dedispersion needs nchan <= 2048 and freq_res <= 4096 in this build");
     const double abw = std::fabs(prm->bw_mhz[0]);
     if (abw <= 0) return fail(B2F_EINVAL, "bw_mhz");
@@ -912,6 +957,7 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     pl->groups_per_slot = (payload + 31) / 32;
     pl->dedisp = dedisp;
     pl->generic = generic;
+    pl->longfft = longfft;
     pl->carry_mode = dedisp || generic;
     pl->bps = (!W && prm->in_nbit == 8) ? 2 : 1;
     pl->smask = pl->carry_mode && pl->bps == 2;
@@ -922,7 +968,11 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
         // submit_job.py:62), half of it on each side plus 10 %, rounded up to a multiple of tscrunch so
         // that every block yields whole output samples
         const int nf = nfilt_half(D);
-        if (2 * nf >= L) { delete pl; return fail(B2F_EUNSUPPORTED, "dispersion smearing exceeds freq_res channel samples (freq_res up to 4096)"); }
+        if (2 * nf >= L) {
+            delete pl;
+            return fail(B2F_EUNSUPPORTED, "dispersion smearing exceeds freq_res channel samples (freq_res up to " + std::to_string(long_cap) + " at nchan " +
+                                              std::to_string(prm->nchan) + ")");
+        }
         pl->nfilt_pos = pl->nfilt_neg = nf;
         pl->keep = L - 2 * nf;
         pl->step = (int64_t)pl->keep * R;
@@ -1121,7 +1171,7 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
             }
         }
     }
-    if (generic) {
+    if (generic && !longfft) {
         auto pass_tables = [](int len) {                 // layout of kg_tw_offset: per outer pass, [q - 1][lo]
             std::vector<float2> t((size_t)len, make_float2(1.f, 0.f));
             const int lg = 31 - __builtin_clz(len);

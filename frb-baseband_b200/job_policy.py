@@ -124,7 +124,9 @@ def coherent_search_plan(dm_max: float | None, fref_mhz: float, if_mhz: float, n
     A channel dedispersed at DM d keeps 8.3 us * |DM - d| * chbw / f_min^3 of smearing at the bottom of the band.  Trials
     `step` apart with step = 2 t_res f_min^3 / (8.3 chbw), at step/2 + k step, leave at most t_res for every DM in
     [0, dm_max].  More than MAX_TRIAL_DMS trials is a ValueError: use fewer channels' worth of time resolution or a lower
-    dm_max."""
+    dm_max.  With few wide channels the largest trial may need overlap-save transforms longer than 4096 points; libb2f
+    takes up to 2^20 / (2 nchan) of them (nchan_if=32 at 1.25 GHz: 52 trials to DM 1500 on 16384 points), while nchan_if=16
+    needs more than 64 trials to DM 1500 and stays a ValueError here."""
     dm_max = UNKNOWN_DM if dm_max is None else float(dm_max)
     if not dm_max > 0:
         raise ValueError(f"dm_max = {dm_max}: must be > 0")

@@ -93,8 +93,11 @@ typedef struct b2f_params {
     int32_t nchan;                 /* channels per IF        (--nchan, digifil -F<nchan>:..)  */
     int32_t freq_res;              /* digifil -F ..:<freq_res>; 0 = reference rule
                                       512 if nchan<=128 else 2*nchan (process_vdif.py:162); with `coherent` the
-                                      dedispersion kernel may lengthen it (next power of two >= 4 nfilt, up to 4096)
-                                      when the smearing does not fit: b2f_geometry.freq_res is what was chosen */
+                                      dedispersion kernel may lengthen it (next power of two >= 4 nfilt, up to 4096,
+                                      and for nchan 8..64 on up to 2^20 / (2 nchan): 65536 at nchan 8, 8192 at
+                                      nchan 64) when the smearing does not fit: b2f_geometry.freq_res is what was
+                                      chosen.  An explicit freq_res above 4096 (other than nchan 4096's 8192) needs
+                                      coherent dedispersion and 2 nchan freq_res <= 2^20 */
     int32_t tscrunch;              /* digifil -t             (--tscrunch)                     */
     int32_t pol_mode;              /* enum b2f_pol_mode                                       */
     int32_t out_nbit;              /* digifil -b: 2, 8, 16, -32 (process_vdif.py:153)         */
@@ -114,7 +117,8 @@ typedef struct b2f_params {
                                       frequency for base2fil's plan                           */
     double dm;                     /* digifil -D dm (process_vdif.py:177-178)                 */
     int32_t coherent;              /* digifil -F nchan:D: in-channel coherent dedispersion by overlap-save (:179-180);
-                                      nchan <= 2048, smearing up to what 4096 points hold */
+                                      nchan <= 2048, smearing up to what 4096 points hold, or for nchan 8..64 up to
+                                      what 2^20 / (2 nchan) points hold */
     int32_t profile;               /* 1: time every kernel launch with CUDA events            */
     void* stream;                  /* cudaStream_t to launch on; NULL = plan-owned stream     */
     int32_t raw_word_bits;         /* 0: frames[i] is the split 2-channel VDIF stream of IF i (what jive5ab's
@@ -135,7 +139,8 @@ typedef struct b2f_params {
     /* ---- coherent dedispersion at several trial DMs in one pass: the spectrum of every overlap-save block is computed once
        and each trial applies its own chirp to it, so one plan writes ndm filterbanks.  Needs coherent = 1 and dm = 0;
        trials finite, >= 0, strictly increasing, the largest > 0.  freq_res, nfilt and the push size follow the largest
-       trial by the single-DM rule, and its refusals apply (smearing beyond 4096 points, nchan 4096). */
+       trial by the single-DM rule, and its refusals apply (smearing beyond 4096 points, or beyond 2^20 / (2 nchan) points
+       for nchan 8..64; nchan 4096). */
     int32_t ndm;                   /* 0: one DM, taken from dm; 1..B2F_MAX_DM: trial DMs dm_trials[0..ndm-1]          */
     double dm_trials[B2F_MAX_DM];
 } b2f_params;
