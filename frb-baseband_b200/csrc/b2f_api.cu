@@ -1044,9 +1044,11 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
         pl->path = eligible ? want : 0;
         // JA98 decode: the round-2 column kernel has its own implementation (levels per block from the frames); every other
         // kernel family (generic, round-1 tuned, dedispersion, raw input) reads levels per window of 512 samples of the
-        // de-framed stream (kj_levels_stream).  The generic kernels address windows from the block start: blocks must start
-        // on multiples of 512 samples.
-        if (prm->decode_mode == B2F_DECODE_JA98 && generic && pl->step % 512) {
+        // de-framed stream (kj_levels_stream).  Its windows count from the first carried sample of each push, so they are
+        // the scan's windows only if blocks start on multiples of 512 samples.  That holds for every shape without
+        // dedispersion (step = M = 512 R on the tuned path); with dedispersion the overlap-save step is keep R, which
+        // at nchan 8..64 need not be a multiple of 512.
+        if (prm->decode_mode == B2F_DECODE_JA98 && pl->step % 512) {
             delete pl;
             return fail(B2F_EUNSUPPORTED, "decode_mode JA98 needs FFT blocks that start on multiples of 512 samples");
         }
