@@ -35,6 +35,7 @@ class Params(C.Structure):
         ("rescale_mode", C.c_int32), ("digi_sigma", C.c_double),
         ("raw_format", C.c_int32), ("reserved0", C.c_int32),
         ("ndm", C.c_int32), ("dm_trials", C.c_double * B2F_MAX_DM),
+        ("remove_delays", C.c_int32), ("delay_ref_mhz", C.c_double),
     ]
 
 
@@ -113,6 +114,7 @@ SYMBOLS = {
     "b2f_wait": (C.c_int, [C.c_void_p, C.c_int64]),
     "b2f_get_params": (C.c_int, [C.c_void_p, C.POINTER(Params)]),
     "b2f_channeliser_path": (C.c_int, [C.c_void_p]),
+    "b2f_get_delays": (C.c_int, [C.c_void_p, C.c_void_p]),
     "b2f_sigproc_header": (C.c_int, [C.POINTER(FilHeaderC), C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "b2f_run_scan": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_char_p), C.c_char_p, C.POINTER(ScanIO),
                                C.POINTER(ScanResult)]),

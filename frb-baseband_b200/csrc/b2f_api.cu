@@ -95,6 +95,16 @@ struct b2f_plan {
     int tsq = 1;
     float* d_Fk = nullptr;
     int64_t Fk_if_stride = 0, fk_pending = 0;
+    // digifil -K (remove_delays, some delay > 0): the row kernels integrate nothing (D = 1) and write channel samples into
+    // d_Fk, a ring of dl_cap rows per (trial, IF) slot; kd_delay_sum adds Du = tscrunch of them at each channel's delay into F.
+    // Logical sample j of the ring (j = 0: the first sample of the next output row) sits at row dl_off + j, minus dl_wrap
+    // where that reaches dl_wrap.  A push that does not fit behind the held samples starts again at row 0 (dl_wrapped);
+    // dl_cap = d_max + Du - 1 + two pushes guarantees it fits there, so nothing is ever moved.
+    bool delays = false, dl_wrapped = false;
+    int Du = 1;
+    int64_t dl_max = 0, dl_cap = 0, dl_off = 0, dl_held = 0, dl_wrap = 0, dl_w = 0;
+    std::vector<int64_t> dl_host;  // delays [trial][if][chan] (remove_delays = 1), for b2f_get_delays
+    int64_t* d_delays = nullptr;
     int kgt_lg = 0;                // generic kernels with compile-time geometry (L = R = 2^kgt_lg), 0 = run-time kernels
     int kgt_cols = 0, kgt_rb = 0, kgt_col_ctas = 0, kgt_row_ctas = 0;
     bool carry_mode = false;       // pushes need not hold whole blocks: unconsumed samples are carried over
@@ -152,9 +162,12 @@ namespace {
 static const int kStatSplit = 64;
 
 // where the row kernels put their rows: straight into F, or behind the rows still waiting in the staging buffer
-inline float* row_dst(const b2f_plan* pl) { return pl->tsq > 1 ? pl->d_Fk : pl->d_F; }
-inline int64_t row_dst_stride(const b2f_plan* pl) { return pl->tsq > 1 ? pl->Fk_if_stride : pl->F_if_stride; }
-inline int64_t row_dst_row0(const b2f_plan* pl) { return pl->tsq > 1 ? pl->fk_pending : pl->rows_off + pl->rows_held; }
+// (with remove_delays: channel samples into the delay ring)
+inline float* row_dst(const b2f_plan* pl) { return pl->tsq > 1 || pl->delays ? pl->d_Fk : pl->d_F; }
+inline int64_t row_dst_stride(const b2f_plan* pl) { return pl->tsq > 1 || pl->delays ? pl->Fk_if_stride : pl->F_if_stride; }
+inline int64_t row_dst_row0(const b2f_plan* pl) {
+    return pl->delays ? pl->dl_w : pl->tsq > 1 ? pl->fk_pending : pl->rows_off + pl->rows_held;
+}
 
 template <class Fn>
 int timed(b2f_plan* pl, int kid, Fn&& fn) {
@@ -322,7 +335,8 @@ void free_plan(b2f_plan* pl) {
     void* bufs[] = {pl->d_compact, pl->d_wmask, pl->d_fstat, pl->d_blkdirty, pl->d_inter, pl->d_colsum,
                     pl->d_eps, pl->d_F, pl->d_mean, pl->d_scale, pl->d_partial, pl->d_tab_g, pl->d_tab_h,
                     pl->d_tab_w, pl->d_tab_r, pl->d_tab_beta, pl->d_counters, pl->d_carry, pl->d_spec, pl->d_chirp, pl->d_tw_col, pl->d_tw_row,
-                    pl->d_tstream, pl->d_fillflag, pl->d_part, pl->d_fsync, pl->d_fprof, pl->d_levels, pl->d_carry_mask, pl->d_levels_stream};
+                    pl->d_tstream, pl->d_fillflag, pl->d_part, pl->d_fsync, pl->d_fprof, pl->d_levels, pl->d_carry_mask, pl->d_levels_stream,
+                    pl->d_delays};
     for (void* b : bufs)
         if (b) cudaFree(b);
     if (pl->d_Fk) cudaFree(pl->d_Fk);
@@ -342,6 +356,9 @@ int init_state(b2f_plan* pl) {
     pl->frames_pushed = 0;
     pl->carry_len = 0;
     pl->fk_pending = 0;
+    pl->dl_off = pl->dl_held = pl->dl_w = 0;
+    pl->dl_wrap = pl->dl_cap;
+    pl->dl_wrapped = false;
     pl->blocks_dirty = 0;
     pl->last_nblk = pl->last_nframes = 0;
     pl->rows_this_interval = 0;
@@ -816,6 +833,80 @@ int sum_rows(b2f_plan* pl, int64_t krows, int64_t rows) {
 }
 }  // namespace
 
+// digifil -K: output row r of slot (trial, IF) = sum of the Du channel samples r Du + k + d_c (k < Du) of the delay ring, added
+// in order k = 0, 1, ...  Threads run over (row, column) with the column fastest and the slot in blockIdx.y, so the CTAs in
+// flight cover a narrow band of rows of one slot: a lane's load touches its own 32-byte sector (neighbouring channels sit at
+// rows d_c apart), and the other channels of that sector are read by later rows while it is still in L2.  Each byte of the
+// ring is read from DRAM about once.
+struct KDParams {
+    const float* Fk;
+    int64_t Fk_stride, off, wrap;  // ring rows per slot, row of logical sample 0, wrap point
+    float* F;
+    int64_t F_stride, row0, nrows;
+    const int64_t* delays;         // [slot][chan]
+    int ncol, N, Du;
+};
+
+static __global__ void __launch_bounds__(256) kd_delay_sum(KDParams p) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= p.nrows * p.ncol) return;
+    const int64_t r = i / p.ncol;
+    const int col = (int)(i - r * p.ncol);
+    const int c = col % p.N;
+    const float* src = p.Fk + blockIdx.y * p.Fk_stride + col;
+    int64_t q = p.off + r * p.Du + p.delays[(int64_t)blockIdx.y * p.N + c];
+    if (q >= p.wrap) q -= p.wrap;
+    float acc = src[q * p.ncol];
+    for (int k = 1; k < p.Du; ++k) {
+        if (++q == p.wrap) q = 0;
+        acc += src[q * p.ncol];
+    }
+    p.F[blockIdx.y * p.F_stride + (p.row0 + r) * p.ncol + col] = acc;
+}
+
+namespace {
+// where this push's channel samples go in the ring (before the row kernels run)
+int delay_place(b2f_plan* pl, int64_t krows) {
+    if (!pl->delays || krows == 0) return 0;
+    int64_t w = pl->dl_off + pl->dl_held;
+    if (!pl->dl_wrapped) {
+        if (w + krows > pl->dl_cap) {
+            pl->dl_wrap = w;
+            pl->dl_wrapped = true;
+            w = 0;
+        }
+    } else {
+        w -= pl->dl_wrap;
+    }
+    if (pl->dl_wrapped && w + krows > pl->dl_off) return fail(B2F_ESTATE, "internal: delay ring overrun");
+    pl->dl_w = w;
+    return 0;
+}
+
+// rows of this push from the ring into F; the consumed samples leave the ring
+int delay_sum(b2f_plan* pl, int64_t krows, int64_t rows) {
+    const int ncol = pl->nprod * pl->N, nslot = pl->ndm * pl->prm.nif;
+    if (rows > 0) {
+        KDParams kd{};
+        kd.Fk = pl->d_Fk; kd.Fk_stride = pl->Fk_if_stride; kd.off = pl->dl_off; kd.wrap = pl->dl_wrap;
+        kd.F = pl->d_F; kd.F_stride = pl->F_if_stride; kd.row0 = pl->rows_off + pl->rows_held; kd.nrows = rows;
+        kd.delays = pl->d_delays; kd.ncol = ncol; kd.N = pl->N; kd.Du = pl->Du;
+        const int64_t n = rows * ncol;
+        int rc = timed(pl, B2F_K_TSUM, [&] { kd_delay_sum<<<dim3((unsigned)((n + 255) / 256), nslot), 256, 0, pl->stream>>>(kd); });
+        if (rc) return rc;
+    }
+    const int64_t used = rows * pl->Du;
+    pl->dl_held += krows - used;
+    pl->dl_off += used;
+    if (pl->dl_wrapped && pl->dl_off >= pl->dl_wrap) {
+        pl->dl_off -= pl->dl_wrap;
+        pl->dl_wrap = pl->dl_cap;
+        pl->dl_wrapped = false;
+    }
+    return 0;
+}
+}  // namespace
+
 extern "C" {
 
 int b2f_version(void) { return B2F_VERSION; }
@@ -936,6 +1027,42 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     if (std::fabs(fps_d - (double)fps) > 1e-6) return fail(B2F_EINVAL, "frames per second is not an integer");
     if (nprod * prm->nchan % 4 || (prm->out_nbit == 2 && (int64_t)prm->nif * nprod * prm->nchan % 4))
         return fail(B2F_EINVAL, "row size");
+    // digifil -K: inter-channel delays [trial][if][chan] in channel samples (b2f.h), refused here before any device call
+    if (prm->remove_delays != 0 && prm->remove_delays != 1) return fail(B2F_EINVAL, "remove_delays must be 0 or 1");
+    if (!prm->remove_delays && prm->delay_ref_mhz != 0.0) return fail(B2F_EINVAL, "delay_ref_mhz needs remove_delays = 1");
+    std::vector<int64_t> dl_table;
+    int64_t dl_max = 0;
+    if (prm->remove_delays) {
+        if (!std::isfinite(prm->dm) || prm->dm < 0) return fail(B2F_EINVAL, "remove_delays needs a finite dm >= 0");
+        double top = -1e300, bottom = 1e300;
+        for (int i = 0; i < prm->nif; ++i) {
+            top = std::max(top, prm->freq_mhz[i] + abw / 2 - abw / (2.0 * prm->nchan));
+            bottom = std::min(bottom, prm->freq_mhz[i] - abw / 2 + abw / (2.0 * prm->nchan));
+        }
+        if (!(bottom > 0)) return fail(B2F_EINVAL, "remove_delays needs every channel centre above 0 MHz");
+        if (!std::isfinite(prm->delay_ref_mhz) || (prm->delay_ref_mhz != 0.0 && prm->delay_ref_mhz < top - 1e-9))
+            return fail(B2F_EINVAL, "delay_ref_mhz must be 0 (the plan's highest channel centre, " + std::to_string(top) +
+                                        " MHz) or a finite frequency at least that high");
+        const double ref = prm->delay_ref_mhz != 0.0 ? prm->delay_ref_mhz : top;
+        const double tsamp0 = prm->nchan / (abw * 1e6);
+        const int nd = std::max(1, prm->ndm);
+        dl_table.resize((size_t)nd * prm->nif * prm->nchan);
+        for (int t = 0; t < nd; ++t) {
+            const double dmt = prm->ndm > 0 ? prm->dm_trials[t] : prm->dm;
+            for (int i = 0; i < prm->nif; ++i) {
+                const double bw = prm->bw_mhz[i];
+                for (int c = 0; c < prm->nchan; ++c) {
+                    const double fc = prm->freq_mhz[i] - bw / 2 + (c + 0.5) * bw / prm->nchan;
+                    const double v = (1.0 / 2.41e-4) * dmt * (1.0 / (fc * fc) - 1.0 / (ref * ref)) / tsamp0;
+                    if (!(v < 1e15)) return fail(B2F_EINVAL, "inter-channel delay beyond 1e15 channel samples");
+                    const int64_t d = std::max<int64_t>(0, llround(v));
+                    dl_table[((size_t)t * prm->nif + i) * prm->nchan + c] = d;
+                    dl_max = std::max(dl_max, d);
+                }
+            }
+        }
+    }
+    const bool delays = dl_max > 0;          // all delays 0 (DM 0): exactly the plan without remove_delays
 
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
@@ -1005,6 +1132,18 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     if (pl->carry_mode) pl->chunk_blocks += 1;                 // carried samples can complete one more block
     pl->chunk_rows = pl->chunk_blocks * pl->keep / D;
     if (tsq > 1) pl->chunk_rows = pl->chunk_rows / tsq + 1;       // a push can complete one more output sample than its share
+    pl->dl_host = dl_table;
+    if (delays) {
+        // the geometry above is the plain plan's; only the kernels' integration factor changes
+        const int64_t P = pl->chunk_blocks * pl->keep;            // channel samples of one push at most
+        pl->delays = true;
+        pl->Du = D_user;
+        pl->D = 1;
+        pl->tsq = 1;
+        pl->dl_max = dl_max;
+        pl->dl_cap = dl_max + D_user - 1 + 2 * P;
+        pl->chunk_rows = (P + D_user - 1) / D_user;               // held samples short of a row + one push
+    }
     const double tsamp = (double)D_user * prm->nchan / (abw * 1e6);
     const double interval = prm->rescale_interval_s > 0 ? prm->rescale_interval_s : 10.0;
     pl->interval_rows = prm->keep_bandpass ? 0 : (int64_t)llround(interval / tsamp);
@@ -1064,7 +1203,7 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
                 pl->f_grid = pl->num_sms;                                  // one 16-warp CTA per SM
                 pl->f_lanes = pl->f_grid * kFWarps / npair;
                 if (pl->f_lanes < 1) pl->path = 0;
-                pl->Dp = std::min(D, 1024 / R);
+                pl->Dp = std::min(pl->D, 1024 / R);
             }
         }
     }
@@ -1097,7 +1236,8 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     const int64_t nbt = (int64_t)nif * pl->chunk_blocks;
     const int nslot = pl->ndm * nif;                        // F / statistics slots: (trial, IF), trial-major
     pl->F_if_stride = pl->F_cap_rows * nprod * pl->N;
-    if (tsq > 1) pl->Fk_if_stride = (pl->chunk_blocks * pl->keep / D + tsq) * nprod * pl->N;
+    if (pl->tsq > 1) pl->Fk_if_stride = (pl->chunk_blocks * pl->keep / D + tsq) * nprod * pl->N;
+    if (pl->delays) pl->Fk_if_stride = pl->dl_cap * nprod * pl->N;
     if (prm->ndm > 0) {
         // what grows with the trials, and the two spectrum-sized buffers, against what the device has free
         const int64_t blocks = pl->batch_blocks > 0 ? std::min<int64_t>(pl->batch_blocks, nbt) : nbt;
@@ -1110,6 +1250,17 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
         if (need > (double)fr) {
             g_err = "ndm = " + std::to_string(prm->ndm) + " trial DMs need " + std::to_string((int64_t)(need / (1 << 20))) + " MiB of device memory, " +
                     std::to_string((int64_t)(fr >> 20)) + " MiB are free: use fewer trials or a smaller chunk_units";
+            return bail(B2F_ENOMEM);
+        }
+    }
+    if (pl->delays) {
+        const double hold = (double)nslot * pl->Fk_if_stride * sizeof(float);
+        size_t fr = 0, tot = 0;
+        CUB(cudaMemGetInfo(&fr, &tot));
+        if (hold > (double)fr) {
+            g_err = "remove_delays holds " + std::to_string((int64_t)hold) + " bytes of channel samples (d_max = " + std::to_string(dl_max) +
+                    " samples plus two pushes, per trial and IF), " + std::to_string((int64_t)fr) +
+                    " bytes are free: use fewer IFs or trials per plan, or a smaller chunk_units";
             return bail(B2F_ENOMEM);
         }
     }
@@ -1133,7 +1284,7 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
             CUB(cudaMalloc(&pl->d_fprof, (size_t)pl->f_grid * kFWarps * 8 * sizeof(unsigned long long)));
             CUB(cudaMemset(pl->d_fprof, 0, (size_t)pl->f_grid * kFWarps * 8 * sizeof(unsigned long long)));
         }
-        if (pl->Dp < D && pl->path == 2) {
+        if (pl->Dp < pl->D && pl->path == 2) {
             pl->part_if_stride = pl->chunk_blocks * (L / pl->Dp) * nprod * pl->N;
             CUB(cudaMalloc(&pl->d_part, (size_t)pl->part_if_stride * nif * sizeof(float)));
         }
@@ -1145,7 +1296,11 @@ int b2f_plan_create(const b2f_params* prm, b2f_plan** out) {
     CUB(cudaMalloc(&pl->d_colsum, (size_t)nbt * R * sizeof(float2)));
     CUB(cudaMalloc(&pl->d_eps, (size_t)nbt * pl->N * sizeof(float2)));
     CUB(cudaMalloc(&pl->d_F, (size_t)pl->F_if_stride * nslot * sizeof(float)));
-    if (tsq > 1) CUB(cudaMalloc(&pl->d_Fk, (size_t)pl->Fk_if_stride * nslot * sizeof(float)));
+    if (pl->tsq > 1 || pl->delays) CUB(cudaMalloc(&pl->d_Fk, (size_t)pl->Fk_if_stride * nslot * sizeof(float)));
+    if (pl->delays) {
+        CUB(cudaMalloc(&pl->d_delays, dl_table.size() * sizeof(int64_t)));
+        CUB(cudaMemcpy(pl->d_delays, dl_table.data(), dl_table.size() * sizeof(int64_t), cudaMemcpyHostToDevice));
+    }
     CUB(cudaMalloc(&pl->d_mean, (size_t)nslot * nprod * pl->N * sizeof(float)));
     CUB(cudaMalloc(&pl->d_scale, (size_t)nslot * nprod * pl->N * sizeof(float)));
     CUB(cudaMalloc(&pl->d_partial, (size_t)nslot * kStatSplit * nprod * pl->N * sizeof(double2)));
@@ -1240,7 +1395,7 @@ int b2f_get_geometry(const b2f_plan* pl, b2f_geometry* g) {
     g->row_bytes = pl->row_bytes;
     g->nprod = pl->nprod;
     g->freq_res = pl->L;
-    g->tsamp_s = (double)pl->D * pl->tsq * pl->N / (std::fabs(pl->prm.bw_mhz[0]) * 1e6);
+    g->tsamp_s = (double)pl->prm.tscrunch * pl->N / (std::fabs(pl->prm.bw_mhz[0]) * 1e6);
     g->unit_blocks = pl->unit_blocks;
     g->interval_rows = pl->interval_rows;
     g->nfilt_pos = pl->nfilt_pos;
@@ -1268,7 +1423,8 @@ int b2f_push(b2f_plan* pl, const void* const* frames, int64_t nframes, int on_de
     const int64_t T = pl->carry_len + nframes * pl->spf;          // samples available per IF (carry + new)
     const int64_t nblk = pl->carry_mode ? (T >= pl->M ? (T - pl->M) / pl->step + 1 : 0) : nframes * pl->spf / pl->M;
     const int64_t krows = nblk * pl->keep / pl->D;                     // rows the kernels write
-    const int64_t rows = pl->tsq > 1 ? (pl->fk_pending + krows) / pl->tsq : krows;
+    int64_t rows = pl->tsq > 1 ? (pl->fk_pending + krows) / pl->tsq : krows;
+    if (pl->delays) rows = pl->dl_held + krows >= pl->dl_max ? (pl->dl_held + krows - pl->dl_max) / pl->Du : 0;   // tail dropped
     if (nblk == 0 && !pl->carry_mode) return 0;
     if (pl->rows_off + pl->rows_held + rows > pl->F_cap_rows && pl->rows_off > 0 && pl->rows_held + rows <= pl->F_cap_rows) {
         // running rescale keeps the rows of an unfinished interval: move them to the front of the buffer, in pieces no
@@ -1285,6 +1441,7 @@ int b2f_push(b2f_plan* pl, const void* const* frames, int64_t nframes, int on_de
     }
     if (pl->rows_off + pl->rows_held + rows > pl->F_cap_rows)
         return fail(B2F_ESTATE, "row buffer full: call b2f_pull before pushing more");
+    if (int rcd = delay_place(pl, krows)) return rcd;
     const size_t fbytes = (size_t)nframes * pl->prm.frame_bytes;
 
     if (!pl->have_base) {
@@ -1356,7 +1513,7 @@ int b2f_push(b2f_plan* pl, const void* const* frames, int64_t nframes, int on_de
             CU(cudaEventRecord(pl->ev_stage_free[pl->stage_idx], pl->stream));
             pl->stage_idx ^= 1;
         }
-        rc = sum_rows(pl, krows, rows);
+        rc = pl->delays ? delay_sum(pl, krows, rows) : sum_rows(pl, krows, rows);
         if (rc) return rc;
         pl->rows_held += rows;
         pl->rows_produced += rows;
@@ -1467,7 +1624,7 @@ int b2f_push(b2f_plan* pl, const void* const* frames, int64_t nframes, int on_de
             if (rc) return rc;
         }
     }
-    rc = sum_rows(pl, krows, rows);
+    rc = pl->delays ? delay_sum(pl, krows, rows) : sum_rows(pl, krows, rows);
     if (rc) return rc;
     pl->rows_held += rows;
     pl->rows_produced += rows;
@@ -1617,6 +1774,14 @@ int b2f_wait(b2f_plan* pl, int64_t ticket) {
 }
 
 int b2f_channeliser_path(const b2f_plan* pl) { return pl ? pl->path : B2F_EINVAL; }
+
+int b2f_get_delays(const b2f_plan* pl, int64_t* out) {
+    if (!pl || !out) return fail(B2F_EINVAL, "null argument");
+    const size_t n = (size_t)pl->ndm * pl->prm.nif * pl->N;
+    if (pl->dl_host.size() == n) std::copy(pl->dl_host.begin(), pl->dl_host.end(), out);
+    else std::fill(out, out + n, (int64_t)0);
+    return 0;
+}
 
 int b2f_get_params(const b2f_plan* pl, b2f_params* out) {
     if (!pl || !out) return fail(B2F_EINVAL, "null argument");

@@ -351,8 +351,17 @@ extern "C" int b2f_run_scan(b2f_plan* pl, int nfiles, const char* const* vdif_pa
         const int64_t A = NB / ub, k = io.part_index, n = io.part_count;
         const int64_t b_lo = A * k / n * ub, b_hi = k == n - 1 ? NB : A * (k + 1) / n * ub;
         const int64_t skip = b_lo * step / spf;                           // exact: b_lo is a multiple of ub
+        // remove_delays: the last own row also reads d_max channel samples further on, i.e. whole blocks beyond b_hi
+        int64_t dl_max = 0;
+        if (prm.remove_delays) {
+            std::vector<int64_t> dl((size_t)g.ndm * prm.nif * prm.nchan);
+            rc = b2f_get_delays(pl, dl.data());
+            if (rc) return rc;
+            for (int64_t d : dl) dl_max = std::max(dl_max, d);
+        }
+        const int64_t b_end = std::min(NB, b_hi + (dl_max + keep - 1) / keep);
         int64_t take = nfr - skip;
-        if (k < n - 1) take = std::min(take, ((b_hi - b_lo - 1) * step + M + spf - 1) / spf);   // includes the overlap halo
+        if (k < n - 1) take = std::min(take, ((b_end - b_lo - 1) * step + M + spf - 1) / spf);   // includes the overlap halo
         if (b_hi <= b_lo) take = 0;
         f0 += skip;
         nfr = std::max<int64_t>(take, 0);

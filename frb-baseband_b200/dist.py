@@ -24,6 +24,13 @@ def rank_if_plan(nif_total: int, world: int, rank: int, freq_lsb0: float, bw: fl
     return ifs, bws, freqs
 
 
+def band_reference_mhz(nif_total: int, freq_lsb0: float, bw: float, nchan: int) -> float:
+    """Centre of the highest channel of base2fil's whole band (the spliced file's fch1): the delay_ref_mhz every rank of an
+    IF-sharded scan passes with remove_delays, so that all ranks align their channels to the same frequency."""
+    top = max(freq_lsb0 + (i - 1) * bw for i in range(1, nif_total + 1))
+    return top + abs(bw) / 2 - abs(bw) / (2 * nchan)
+
+
 def gather_splice(local_rows, world: int, rank: int, dst: int = 0, group=None, out=None):
     """Gather every rank's [rows, tile_bytes] uint8 tensor to `dst` and lay the tiles out in
     splice order: highest sky frequency first, i.e. rank world-1's tile leftmost

@@ -60,6 +60,8 @@ class PlanConfig:
     fft_normalised: bool = False             # D4
     rescale_mode: int = 0                    # 0 digifil -c (first interval, frozen), 1 running (D8)
     digi_sigma: float = 0.0                  # D9: 0 = 6 sigma
+    remove_delays: bool = False              # digifil -K: inter-channel dispersion delays at dm (or each trial) removed
+    delay_ref_mhz: float = 0.0               # -K reference frequency; 0 = the plan's highest channel centre
     extra: dict = field(default_factory=dict)
 
 
@@ -119,6 +121,8 @@ class Plan:
         p.fft_normalised = int(cfg.fft_normalised)
         p.rescale_mode = cfg.rescale_mode
         p.digi_sigma = cfg.digi_sigma
+        p.remove_delays = int(cfg.remove_delays)
+        p.delay_ref_mhz = float(cfg.delay_ref_mhz)
         self.if_order = list(order)
         self.freq_mhz = list(freq)
         self._h = C.c_void_p()
@@ -285,6 +289,13 @@ class Plan:
         s = np.ascontiguousarray(scale, np.float32).reshape(-1)
         assert m.size == s.size == self.ndm * self.nif * self.nprod * self.cfg.nchan
         _lib.check(_lib.lib().b2f_set_rescale(self._h, m.ctypes.data, s.ctypes.data))
+
+    def delays(self) -> np.ndarray:
+        """Inter-channel delays the plan removes (remove_delays), in channel samples: int64 [ndm, nif, nchan] in plan IF
+        order and natural channel order (ndm = 1 without trials); zeros without remove_delays."""
+        out = np.empty((self.ndm, self.nif, self.cfg.nchan), np.int64)
+        _lib.check(_lib.lib().b2f_get_delays(self._h, out.ctypes.data))
+        return out
 
     def kernel_times(self) -> dict:
         out = {}

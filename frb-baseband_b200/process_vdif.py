@@ -52,6 +52,9 @@ _CLI = [
                                   help="extension: with N >= 2, coherent dedispersion at the N trial DMs coherent_dm + k "
                                        "coherent_dmstep in one pass, one <stem>_DM<dm>.fil per trial (%(default)s)"), _D),
     (("--coherent_dmstep",), dict(type=float, default=0.0, help="extension: DM step of the coherent trials"), _D),
+    (("--remove_delays",), dict(action="store_true",
+                                help="extension: also remove the inter-channel dispersion delays at the coherent DM (or each "
+                                     "trial DM), aligned to the top channel (digifil -K)"), _D),
     (("--do_prepdata",), dict(action="store_true", help="run PRESTO prepdata/prepsubband afterwards"), _P),
     (("--ncpus",), dict(type=int, default=1, help="1: prepdata, >1: prepsubband"), _P),
     (("--dm",), dict(type=float, default=None, help="DM for prepdata (default: psrcat)"), _P),
@@ -164,9 +167,11 @@ def trial_output_paths(hdr, fil_out_dir, dm_trials):
 
 
 def run_digifil(hdr, fil_out_dir=None, start=1, nsecs=120, nchan=128, overwrite=False, pol=2, nbit=8,
-                tscrunch=1, nthreads=1, dm=0.0, coherent=False, keepBP=False, device=0, dm_trials=None):
+                tscrunch=1, nthreads=1, dm=0.0, coherent=False, keepBP=False, device=0, dm_trials=None, remove_delays=False):
     """Baseband -> filterbank for the subband described by `hdr`; returns the .fil path.  With `dm_trials` (a list of
-    DMs) one pass writes a coherently dedispersed filterbank per trial and the list of their paths is returned."""
+    DMs) one pass writes a coherently dedispersed filterbank per trial and the list of their paths is returned.
+    `remove_delays` (digifil -K): the inter-channel delays at `dm` (or each trial DM) are removed as well; with
+    coherent=False that is incoherent dedispersion alone."""
     if dm_trials is not None:
         fils = trial_output_paths(hdr, fil_out_dir, dm_trials)
         for f in fils:
@@ -193,9 +198,11 @@ def run_digifil(hdr, fil_out_dir=None, start=1, nsecs=120, nchan=128, overwrite=
     dedisp = "D -D {0}".format(dm) if (coherent and dm > 0) else reference_freq_res(nchan)
     if dm_trials is not None:
         dedisp = "D -D {0}".format(",".join("{0:.2f}".format(d) for d in dm_trials))
-    print("running b2f -b{0} -S{1} -T{2} -t {3} -o {4} {5} pol={6} -F{7}:{8}{9} (libb2f.so, cuda:{10})".format(
+    if remove_delays and not (coherent and dm > 0) and dm_trials is None:
+        dedisp = "{0} -D {1}".format(dedisp, dm)
+    print("running b2f -b{0} -S{1} -T{2} -t {3} -o {4} {5} pol={6} -F{7}:{8}{9}{10} (libb2f.so, cuda:{11})".format(
         nbit, start, nsecs, tscrunch, " ".join(fil) if dm_trials is not None else fil, hdr, pol, nchan, dedisp,
-        " -I0" if keepBP else "", device))
+        " -K" if remove_delays else "", " -I0" if keepBP else "", device))
     try:
         with open(datafile, "rb") as src:
             info = vdif.parse_header(src.read(32))
@@ -207,6 +214,7 @@ def run_digifil(hdr, fil_out_dir=None, start=1, nsecs=120, nchan=128, overwrite=
                          frame_bytes=info.frame_bytes, header_bytes=info.header_bytes, keep_bandpass=keepBP,
                          device=device, dm=float(dm), coherent=bool(coherent and (dm > 0.0 or dm_trials is not None)),
                          dm_trials=None if dm_trials is None else [float(d) for d in dm_trials],
+                         remove_delays=bool(remove_delays),
                          # the reference passes -2 (:157,160): DSPSR's dynamic 2-bit levels; this build defaults to the
                          # static optimal levels, B2F_DECODE_MODE=ja98 selects the reference-faithful unpacker
                          decode_mode=_lib.DECODE_JA98 if os.environ.get("B2F_DECODE_MODE", "").lower() == "ja98" else _lib.DECODE_STATIC)
@@ -267,7 +275,7 @@ def main(argv=None):
         raise InputError("--do_prepdata takes one filterbank: not with --coherent_numdms >= 2")
     fil = run_digifil(hdr, a.fil_out_dir, a.start, a.nsec, a.nchan, overwrite=a.force, pol=a.pol, nbit=a.nbit,
                       tscrunch=a.tscrunch, nthreads=a.nthreads, keepBP=a.keepBP, device=a.device,
-                      dm=a.coherent_dm, coherent=a.coherent_dm > 0.0, dm_trials=trials)
+                      dm=a.coherent_dm, coherent=a.coherent_dm > 0.0, dm_trials=trials, remove_delays=a.remove_delays)
     if a.do_prepdata:
         prepdata(fil, a.dm if a.dm is not None else psr_info(a.psrname)[2], zerodm=a.nozerodm, clip=a.clip,
                  dm2=a.dm2, dmstep=a.dmstep, ncpus=a.ncpus)

@@ -143,6 +143,18 @@ typedef struct b2f_params {
        for nchan 8..64; nchan 4096). */
     int32_t ndm;                   /* 0: one DM, taken from dm; 1..B2F_MAX_DM: trial DMs dm_trials[0..ndm-1]          */
     double dm_trials[B2F_MAX_DM];
+    /* ---- digifil -K: remove the inter-channel dispersion delays after detection (DSPSR's SampleDelay; recalled, not pinned).
+       Channel c of IF i, sky centre f_c = freq_mhz[i] - bw/2 + (c + 1/2) bw/nchan (bw signed), is delayed by
+       d_c = llround(DM (1/2.41e-4 s MHz^2) (f_c^-2 - f_ref^-2) / tsamp0) channel samples, tsamp0 = nchan/|bw| us, at the DM of
+       dm (with or without coherent dedispersion) or of each trial.  Output row r sums channel samples r D + k + d_c, k < D
+       (D = tscrunch): rows are aligned to the arrival time at f_ref, the rescale statistics come from the delayed rows, and a
+       scan of K0 channel samples yields floor((K0 - d_max) / D) rows (the tail is dropped; d_max over every IF and trial).
+       All delays 0 (DM 0) runs exactly as remove_delays = 0.  Otherwise the plan holds about d_max + two pushes of channel
+       samples per (trial, IF): d_max |bw| 4 B nprod nif ndm and more (B2F_ENOMEM names the bytes when that does not fit). */
+    int32_t remove_delays;         /* 0 or 1                                                                         */
+    double delay_ref_mhz;          /* f_ref; 0 = centre of the plan's highest channel (the fch1 b2f_run_scan writes); else
+                                      finite and >= that centre.  A plan holding some IFs of a wider band (one rank of an
+                                      IF-sharded scan) passes the band's fch1 so that all ranks align to one frequency   */
 } b2f_params;
 
 typedef struct b2f_geometry {
@@ -183,7 +195,8 @@ enum b2f_kernel_id {
     B2F_K_DECODE = 6,              /* stand-alone decode (tests / roofline)                   */
     B2F_K_DEDISP = 7,              /* un-mix + chirp + backward FFT + overlap discard + detect */
     B2F_K_FUSED = 8,               /* decode + column pass + row pass + detection in one persistent kernel */
-    B2F_K_TSUM = 9,                /* sum of partial rows when tscrunch spans the rows of several warps */
+    B2F_K_TSUM = 9,                /* sum of partial rows when tscrunch spans the rows of several warps; with remove_delays
+                                      the delay + integration kernel kd_delay_sum                                     */
     B2F_K_COUNT = 10
 };
 
@@ -248,6 +261,10 @@ int b2f_channeliser_path(const struct b2f_plan* plan);
 
 /* The parameters the plan was created with (freq_res resolved to its effective value). */
 int b2f_get_params(const struct b2f_plan* plan, b2f_params* out);
+
+/* The inter-channel delays the plan removes (remove_delays), in channel samples: ndm * nif * nchan values (ndm = 1 without
+ * trials), trial-major, plan IF order, natural channel order; all 0 without remove_delays. */
+int b2f_get_delays(const struct b2f_plan* plan, int64_t* out);
 
 /* ---- file level: what one `digifil` process per IF plus `splice` do with files ------------------------------- */
 
